@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark: Mrays/s & ms/frame, complex.txt at 1920x1080 depth 5.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one full frame of the hot path (camera rays -> closest hit -> Phong + shadow rays
@@ -256,6 +256,23 @@ def main_reference(args, rank):
     return 0
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_frame(out_dir, frame):
+    """Writes the [H, W, 3] frame of the last timed step as <out_dir>/rgb.npy (float32).  A frame larger than
+    DUMP_BYTES is cut to a fixed, seeded sample of whole rows; their indices go to <out_dir>/rgb_rows.npy (float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    a = frame.cpu().numpy().astype(np.float32)
+    h, w, _ = a.shape
+    if a.nbytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(h, DUMP_BYTES // (w * 3 * 4 + 8), replace=False))
+        np.save(os.path.join(out_dir, "rgb_rows.npy"), rows.astype(np.float64))
+        a = a[rows]
+    np.save(os.path.join(out_dir, "rgb.npy"), a)
+
+
 # -------------------------------------------------------------------------------------------------
 def measure_extra(torch, dist, rtb200, local_rank, rank, n, workload, gather, steps=8, warmup=3):
     """N > 1: a short device-timed run of ANOTHER BASELINE config in the same process group (the 8-GPU config the
@@ -382,6 +399,9 @@ def main_b200(args, rank, local_rank, world):
         step_device()
         ev[k][1].record(stream)
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        # before the barrier: in peer mode the other ranks may render into rank 0's frame once they pass it
+        dump_frame(args.dump_outputs, full if n > 1 else part[:H * W * 3].view(H, W, 3))
     if n > 1:
         dist.barrier()
     # kernels per frame, counted in the steady state the timed loop ran in (the library picks the number of wavefront
@@ -609,10 +629,17 @@ def main_b200(args, rank, local_rank, world):
     return 0
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be >= 1")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=300)
+    ap.add_argument("--steps", type=positive_int, default=300, help="timed steps (frames)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -620,7 +647,11 @@ def main():
     ap.add_argument("--accel", type=int, default=None, help="0 auto, 1 table walks, 2 LBVH (rt_set_option accel)")
     ap.add_argument("--no-extra", action="store_true", help="N > 1: skip the extra_workloads block (config 4)")
     ap.add_argument("--gather", default="peer", choices=["peer", "nccl"], help="N > 1: how the bands reach rank 0")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of the last timed step to DIR/rgb.npy (float32), for comparing two builds")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm keeps no frame")
     global SCENE, W, H, DEPTH, WORKLOAD
     _, W, H, DEPTH, WORKLOAD = WORKLOADS[args.workload]
 
@@ -641,6 +672,8 @@ def main():
             cmd += ["--no-extra"]
         if args.no_cpu_baseline:
             cmd += ["--no-cpu-baseline"]
+        if args.dump_outputs:
+            cmd += ["--dump-outputs", os.path.abspath(args.dump_outputs)]
         return subprocess.call(cmd)
     return main_b200(args, rank, local_rank, world)
 
