@@ -794,12 +794,13 @@ __device__ __forceinline__ void closest_shared_culled(const Tab T, int npairs, c
 // bound of the true centre projection), q = |X|^2 - rho' (>= 0 => origin strictly outside),
 // D' = tu^2 - q.  A sphere is skipped when D' < 0, or when it lies behind an origin that is outside
 // it (tu < 0 and q >= 0): that removes the sphere the ray just left without any extra arithmetic.
-template <int NR>
+// kIds: the walk covers the pairs ids[0..npairs) (ascending, npairs even) instead of 0..npairs (closest_general_culled).
+template <int NR, bool kIds = false>
 __device__ __forceinline__ void closest_general(const float4 *__restrict__ pairs, int npairs, int N, const float (&ox)[NR],
                                                 const float (&oy)[NR], const float (&oz)[NR], const float (&dx)[NR],
                                                 const float (&dy)[NR], const float (&dz)[NR], const bool (&live)[NR], float d64,
                                                 float gS2, float dtmax, const double4 *sph64, const RaySrc (&src)[NR],
-                                                Best (&best)[NR], const bool coop = false) {
+                                                Best (&best)[NR], const bool coop = false, const unsigned short *ids = nullptr) {
   const float kInfl = 1.0f + 24.0f * 5.9604645e-8f;
   float2 nox[NR], noy[NR], noz[NR], idx2[NR], idy2[NR], idz2[NR];
   const float2 dtm = make_float2(dtmax, dtmax);
@@ -823,7 +824,8 @@ __device__ __forceinline__ void closest_general(const float4 *__restrict__ pairs
     for (int p = p0; p < p0 + np; p += 2) {
 #pragma unroll
       for (int k = 0; k < 2; k++) {
-        const float4 A = pairs[2 * (p + k)], B = pairs[2 * (p + k) + 1];
+        const int pk = kIds ? (int)ids[p + k] : p + k;
+        const float4 A = pairs[2 * pk], B = pairs[2 * pk + 1];
         const float2 CX = make_float2(A.x, A.y), CY = make_float2(A.z, A.w), CZ = make_float2(B.x, B.y);
         const float2 NR_ = make_float2(-B.z, -B.w);
 #pragma unroll
@@ -843,12 +845,108 @@ __device__ __forceinline__ void closest_general(const float4 *__restrict__ pairs
       while (__any_sync(kFull, fr != 0u)) {
         if (fr != 0u) {
           const int bit = 31 - __clz(fr);
-          const int pi = p0 + np - 1 - bit;
+          const int pi = kIds ? (int)ids[p0 + np - 1 - bit] : p0 + np - 1 - bit;
           fr &= ~(1u << bit);
           best[r] = slow_closest_general(best[r], pairs, pi, N, ox[r], oy[r], oz[r], dx[r], dy[r], dz[r], d64, gS2, sph64, src[r]);
         }
       }
     }
+  }
+}
+
+// The same walk with bundle culling (general table in shared memory; k_closest1 takes 64 consecutive rays of the
+// tile-ordered level-1 queue, a strip of neighbouring level-0 tiles, so its rays leave a small region in similar directions).  Bound of the bundle: its directions by the cone
+// of warp_cone (axis a, cos/sin theta), its FP32 origins by a ball (centre m = one live ray's origin, radius rb = the
+// largest |o - m|, rounded up).  Per pair, each sphere is tested once for the whole warp; a pair is dropped when neither
+// sphere can be flagged by the filter above for ANY ray of the bundle, so the surviving pairs -- ascending, in the warp's
+// ids[] -- are flagged and decided exactly as in the full walk, in the same order (same hits, same FP64 evaluations).
+//
+// Margin argument (u = 2^-24; X = c - o with the FP32 table centre c and FP32 origin o taken as exact reals, T = X.d,
+// L = |m - c| + rb >= |X|):
+//   * tu - T <= Dl = dtmax + 64u L: the filter's tu = fl(X).d(1 + 24u) + dtmax is an upper bound of T by construction;
+//     fl(X) (u|X|), the inflated direction (25u |X|) and three FMA roundings add at most 32u |X| more.
+//   * q >= |X|^2 (1 - 8u) - rho' (1 + 8u)   (fl(X) and three FMA roundings).
+//   * |d| = 1 +- 3u (FP32 of an exact unit vector): the distance of c from the line is h^2 = |X|^2 - T^2 / |d|^2
+//     <= |X|^2 - T^2 + 7u L^2.
+//   Flagged with T >= 0 (tu >= 0, tu^2 >= q): h^2 <= rho' (1 + 8u) + 2 L Dl + Dl^2 + 15u L^2 <= Re^2 with
+//     Re^2 = rho' (1 + 16u) + 2 L Dl + Dl^2 + 64u L^2: the FORWARD ray from o passes within Re of c.
+//   Flagged with T < 0: then 0 <= tu < Dl, so |X|^2 <= Re^2: o lies within Re of c.  (Flagged because q < 0: the same.)
+//   Shift by o - m (|o - m| <= rb): the forward ray from m with the same direction meets the ball B(c, R2), R2 = Re + rb.
+//   m outside that ball (|c - m| = dist > R2): the directions from m that meet it form a cone of half-angle alpha around
+//   (c - m) / dist, sin alpha = R2 / dist; it meets the bundle's cone iff angle(a, c - m) <= theta + alpha (theta <= 60,
+//   alpha < 90 degrees: cos is monotonic there), i.e. (c - m).a >= cos(theta) sqrt(dist^2 - R2^2) - sin(theta) R2.
+//   A sphere is culled when that fails by more than 2e-5 (dist + R2): >= 100x the FP32 errors of this test itself (the
+//   rounding of c - m, the dot product, dist; cos theta is already lowered and sin theta raised by warp_cone, R2 is rounded
+//   up, the square root rounded down).  So a culled sphere is rejected by the filter for every ray of the bundle.
+// Only the forward ray matters: the filter rejects a sphere behind an origin outside it (the tangent-behind case of
+// include/sphere.h:37 is not reproduced by the general filter in the first place, DESIGN.md section 4).
+// ids: this warp's kGenIds 16-bit slots; survivors are walked in batches of at most kGenIds - 1 (+1: a culled pair pads
+// an odd count to the even length the packed loop needs -- it is rejected for every ray, so its bit never drains).
+constexpr int kGenIds = 96;
+template <int NR>
+__device__ __forceinline__ void closest_general_culled(const float4 *__restrict__ pairs, int npairs, int N, const float (&ox)[NR],
+                                                       const float (&oy)[NR], const float (&oz)[NR], const float (&dx)[NR],
+                                                       const float (&dy)[NR], const float (&dz)[NR], const bool (&live)[NR], float d64,
+                                                       float gS2, float dtmax, const double4 *sph64, const RaySrc (&src)[NR],
+                                                       Best (&best)[NR], unsigned short *ids, unsigned &c_cand, unsigned &c_walks) {
+  const Cone cone = warp_cone<NR>(dx, dy, dz, live);
+  if (!cone.ok) { closest_general<NR>(pairs, npairs, N, ox, oy, oz, dx, dy, dz, live, d64, gS2, dtmax, sph64, src, best); return; }
+  c_walks++;
+  const int lane = threadIdx.x & 31;
+  // the ball: centre = the origin of one live ray (cone.ok: the warp has one), radius rounded up
+  bool any = false;
+  float mx = 0.f, my = 0.f, mz = 0.f;
+#pragma unroll
+  for (int r = NR - 1; r >= 0; r--)
+    if (live[r]) { any = true; mx = ox[r]; my = oy[r]; mz = oz[r]; }
+  const int ml = __ffs(__ballot_sync(kFull, any)) - 1;
+  mx = __shfl_sync(kFull, mx, ml); my = __shfl_sync(kFull, my, ml); mz = __shfl_sync(kFull, mz, ml);
+  float rb = 0.f;
+#pragma unroll
+  for (int r = 0; r < NR; r++)
+    if (live[r]) {
+      const float ex = __fsub_rn(ox[r], mx), ey = __fsub_rn(oy[r], my), ez = __fsub_rn(oz[r], mz);
+      rb = fmaxf(rb, __fsqrt_ru(__fmaf_ru(ez, ez, __fmaf_ru(ey, ey, __fmul_ru(ex, ex)))));
+    }
+  rb = __fmul_ru(__uint_as_float(__reduce_max_sync(kFull, __float_as_uint(rb))), 1.00001f);   // (non-negative: bit order)
+  const float u = 5.9604645e-8f;
+  auto keep = [&](float cx, float cy, float cz, float rho) -> bool {
+    const float wx = __fsub_rn(cx, mx), wy = __fsub_rn(cy, my), wz = __fsub_rn(cz, mz);
+    const float d2 = fmaf(wz, wz, fmaf(wy, wy, wx * wx)), dist = sqrtf(d2);
+    const float Lx = __fadd_ru(__fmul_ru(dist, 1.0001f), rb);
+    const float Dl = __fmaf_ru(64.0f * u, Lx, dtmax);
+    const float re2 = __fmaf_ru(Dl, Dl, __fmaf_ru(__fmul_ru(2.0f, Lx), Dl, __fmaf_ru(__fmul_ru(64.0f * u, Lx), Lx, __fmul_ru(rho, 1.0f + 16.0f * u))));
+    const float R2 = __fadd_ru(__fmul_ru(__fsqrt_ru(re2), 1.00001f), rb);
+    const float R22 = __fmul_ru(R2, R2), d2lo = __fmul_rd(d2, 0.99998f);
+    if (!(d2lo > R22)) return true;                                // (written so that a NaN keeps the sphere)
+    const float wa = fmaf(wz, cone.az, fmaf(wy, cone.ay, wx * cone.ax));
+    return wa >= cone.cth * __fsqrt_rd(__fsub_rd(d2lo, R22)) - cone.sth * R2 - 2e-5f * (dist + R2);
+  };
+  const unsigned lt = (1u << lane) - 1u;
+  int n = 0, spare = 0;
+#pragma unroll 1
+  for (int base = 0; base < npairs; base += 32) {
+    const int p = base + lane;
+    bool k = false;
+    if (p < npairs) {
+      const float4 A = pairs[2 * p], B = pairs[2 * p + 1];
+      k = (2 * p < N && keep(A.x, A.z, B.x, B.z)) || (2 * p + 1 < N && keep(A.y, A.w, B.y, B.w));
+    }
+    const unsigned km = __ballot_sync(kFull, k), cm = __ballot_sync(kFull, p < npairs && !k);
+    if (k) ids[n + __popc(km & lt)] = (unsigned short)p;
+    n += __popc(km);
+    if (cm) spare = base + 31 - __clz(cm);
+    if (n + 33 <= kGenIds && base + 32 < npairs) continue;
+    // (the batch saw whole 32-pair rounds or ended at npairs, a multiple of kGroupPairs: an even number of pairs, so an odd
+    // n means that one of them was culled, and `spare` names a culled pair)
+    c_cand += 2u * (unsigned)n;                                     // (spheres, as the level-0 counts)
+    if (n & 1) { if (lane == 0) ids[n] = (unsigned short)spare; n++; }
+    __syncwarp();
+    if (n > 0) {
+      closest_general<NR, true>(pairs, n, N, ox, oy, oz, dx, dy, dz, live, d64, gS2, dtmax, sph64, src, best, false, ids);
+      __syncwarp();
+    }
+    n = 0;
   }
 }
 

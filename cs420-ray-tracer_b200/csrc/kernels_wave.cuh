@@ -39,6 +39,8 @@ namespace rtf {
 // A camera-ray hit (level 0) has no queue record, carries weight 1 and no colour yet: there the words of (vy, vz), (src, wt)
 // and (ar, ag) hold the EXACT unit direction of the camera ray as three doubles (finish_hit / hit_d0x..z: k_closest0 has it;
 // the shading pass would otherwise redo its two FP64 normalisations for every hit that reflects); view direction = -(float)d0.
+// The word of vx holds, for a camera-ray hit whose path continues, its rank among the reflected rays of its 16x4 tile in
+// slot order (k_closest0): k_shade stores the reflected ray at the tile's offset + rank (tile-ordered level-1 queue).
 // (Plain fields and register-level bit casts, not a union: the record keeps moving as five 128-bit words.)
 struct __align__(16) HitRec {      // 80 bytes
   double px, py, pz;               // exact FP64 hit point (src/main.cpp:32)
@@ -53,6 +55,7 @@ struct __align__(16) HitRec {      // 80 bytes
 __device__ __forceinline__ double hit_d0x(const HitRec &h) { return __hiloint2double(__float_as_int(h.vz), __float_as_int(h.vy)); }
 __device__ __forceinline__ double hit_d0y(const HitRec &h) { return __hiloint2double(__float_as_int(h.wt), (int)h.src); }
 __device__ __forceinline__ double hit_d0z(const HitRec &h) { return __hiloint2double(__float_as_int(h.ag), __float_as_int(h.ar)); }
+__device__ __forceinline__ unsigned hit_ray_rank(const HitRec &h) { return __float_as_uint(h.vx); }
 static_assert(sizeof(HitRec) == 80, "hit record layout");
 
 struct WaveArgs {
@@ -73,6 +76,9 @@ struct WaveArgs {
   unsigned int *ctl, *ctl_next;
   RayRec *queue[2];
   unsigned int *shade_done;        // per chunk of hits: (chunk, light) items finished so far (self-resetting)
+  // per level-0 tile (tile order): the number of its reflected rays (written by k_closest0 for every tile, so never
+  // cleared), turned in place into the position of its first ray in the level-1 queue by CTA 0 of the level-0 k_shadow
+  unsigned int *tile_ray;
 };
 
 // Control words (u32) of one frame: [0] tile counter, [4] grid-barrier arrivals, [5] error word; per level k <= 33: tail
@@ -146,8 +152,8 @@ __device__ __noinline__ void flush_counts(unsigned long long *counters, int leve
   }
 }
 
-// Exact t of the winner + hit record (out of line: FP64 heavy, once per hit ray)
-__device__ __noinline__ bool finish_hit(const FastArgs &a, Best b, RaySrc src, unsigned pix, unsigned srcidx, float wt, float ar, float ag,
+// Exact t of the winner + hit record (out of line: FP64 heavy, once per hit ray); returns the sphere hit, -1 = none
+__device__ __noinline__ int finish_hit(const FastArgs &a, Best b, RaySrc src, unsigned pix, unsigned srcidx, float wt, float ar, float ag,
                                         float ab, HitRec *out, unsigned *viol, unsigned *nfp64) {
   const ExactRay e = exact_ray(src);
   double t = b.t;
@@ -155,7 +161,7 @@ __device__ __noinline__ bool finish_hit(const FastArgs &a, Best b, RaySrc src, u
   if (!ok) { (*nfp64)++; ok = exact_sphere(a.r.sph64, b.idx, e.o, e.d, e.a, t) && t < 1e20; }
   int bi = b.idx;
   if (!ok) { (*viol)++; bi = exact_bruteforce(a.r.sph64, a.N, e.o, e.d, e.a, t); }
-  if (bi < 0) return false;
+  if (bi < 0) return -1;
   const HitGeom g = hit_geometry(a.r.sph64, bi, e.o, e.d, t);
   // (the words of the record are formed first and stored unconditionally, in order: five 128-bit stores)
   float vx = -(float)e.d.x, vy = -(float)e.d.y, vz = -(float)e.d.z;   // view_dir = -d up to rounding (src/main.cpp:38)
@@ -169,7 +175,7 @@ __device__ __noinline__ bool finish_hit(const FastArgs &a, Best b, RaySrc src, u
   out->nx = g.nx; out->ny = g.ny; out->nz = g.nz;
   out->vx = vx; out->vy = vy; out->vz = vz;
   out->idx = bi; out->pix = pix; out->src = srcidx; out->wt = wt; out->ar = ar; out->ag = ag; out->ab = ab; out->pad = 0;
-  return true;
+  return bi;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -350,15 +356,19 @@ __device__ __forceinline__ void closest0_body(const WaveArgs &w, const Lvl &lv, 
     hit_block(w, lv.hit_count, hm0, hm1, hslot);
     // a whole tile with a hit block: the shading pass stores it (tile_path)
     const bool deferred = defer_mixed && (hm0 | hm1) != 0u && tx0 + kWTileW <= W && ty0 + kWTileH <= rows;
+    bool cont[2];                                    // the hit's path continues (shade_one's test): a level-1 ray
 #pragma unroll
     for (int r = 0; r < 2; r++) {
       bool hit = false;
+      cont[r] = false;
       if (live[r]) {
         c_closest++; c_fp64 += best[r].nfp64;
         if (best[r].idx >= 0) {
           HitRec *rec = w.hits + hslot[r];
-          hit = finish_hit(a, best[r], src[r], pix[r], 0u, 1.0f, 0.f, 0.f, 0.f, rec, &c_viol, &c_fp64);
+          const int hi = finish_hit(a, best[r], src[r], pix[r], 0u, 1.0f, 0.f, 0.f, 0.f, rec, &c_viol, &c_fp64);
+          hit = hi >= 0;
           if (!hit) { rec->idx = -1; rec->pix = pix[r]; }   // (filter violation resolved to a miss: dead slot)
+          else cont[r] = depth > 1 && __ldg(&a.r.matx[hi]).y > 0.5f;
           if (a.r.hit_idx) a.r.hit_idx[(size_t)pix[r] * depth] = hit ? rec->idx : -1;
         } else if (a.r.hit_idx) a.r.hit_idx[(size_t)pix[r] * depth] = -1;
       }
@@ -374,6 +384,13 @@ __device__ __forceinline__ void closest0_body(const WaveArgs &w, const Lvl &lv, 
       } else if (sky) {
         write_final(a.r, pix[r], skyc.r, skyc.g, skyc.b);
       }
+    }
+    {
+      // the tile's reflected rays: their count, and each one's rank in slot order (hit_block: the r = 0 hits, then r = 1)
+      const unsigned k0 = __ballot_sync(kFull, cont[0]), k1 = __ballot_sync(kFull, cont[1]), lt = (1u << lane) - 1u;
+      if (cont[0]) w.hits[hslot[0]].vx = __uint_as_float((unsigned)__popc(k0 & lt));
+      if (cont[1]) w.hits[hslot[1]].vx = __uint_as_float((unsigned)(__popc(k0) + __popc(k1 & lt)));
+      if (lane == 0 && tile_ok) w.tile_ray[tile] = (unsigned)(__popc(k0) + __popc(k1));
     }
     if (!kBytes) continue;                           // float / remapped output: only finished pixels are written
     __syncwarp();
@@ -417,15 +434,18 @@ __global__ void __launch_bounds__(kThreads, RT_CLOSEST0_CTAS) k_closest0(const W
 
 // ---------------------------------------------------------------------------------------------
 // LEVEL >= 1 closest hit: reflected rays from the RayRec queue, 64 per warp fetch, two per lane.
-// gen: the general table (shared memory when staged)
-template <bool kBvh>
-__device__ __forceinline__ void closest1_body(const WaveArgs &w, const Lvl &lv, const float4 *gen) {
+// gen: the general table (shared memory when staged); kCull (gen staged): bundle-culled walk, survivors listed in the
+// header's per-warp staging area (unused in this kernel: kGenIds 16-bit slots of its 192 bytes)
+template <bool kBvh, bool kCull = false>
+__device__ __forceinline__ void closest1_body(const WaveArgs &w, const Lvl &lv, const float4 *gen, unsigned char *smem = nullptr) {
   const FastArgs &a = w.f;
   const unsigned nq = __ldcg(lv.q_in_count);
   if (nq == 0u) return;
   const int lane = threadIdx.x & 31, depth = a.r.max_depth, level = lv.level;
-  unsigned c_closest = 0, c_hits = 0, c_fp64 = 0, c_viol = 0;
+  unsigned c_closest = 0, c_hits = 0, c_fp64 = 0, c_viol = 0, c_cand = 0, c_walks = 0;
   const RayRec *qin = lv.q_in;
+  static_assert(kGenIds * 2 <= kWTileH * kWTileW * 3, "survivor list in the header's per-warp staging area");
+  unsigned short *ids = kCull ? reinterpret_cast<unsigned short *>(smem + 64 + (threadIdx.x >> 5) * (kWTileH * kWTileW * 3)) : nullptr;
   // few rays (deep levels): one ray per lane, so that twice as many warps share the work
   const bool two = nq >= gridDim.x * (unsigned)kWarps * 64u * a.two_mult;
   const unsigned per = two ? 64u : 32u;
@@ -458,6 +478,9 @@ __device__ __forceinline__ void closest1_body(const WaveArgs &w, const Lvl &lv, 
 #pragma unroll 1
       for (int r = 0; r < 2; r++)
         if (live[r]) best[r] = bvh_closest_general(a, gen, ox[r], oy[r], oz[r], dx[r], dy[r], dz[r], src[r]);
+    } else if (kCull) {
+      closest_general_culled<2>(gen, a.npairs, a.N, ox, oy, oz, dx, dy, dz, live, a.d64, a.gS2, a.g_dtmax, a.r.sph64, src, best, ids,
+                                c_cand, c_walks);
     } else {
       closest_general<2>(gen, a.npairs, a.N, ox, oy, oz, dx, dy, dz, live, a.d64, a.gS2, a.g_dtmax, a.r.sph64, src, best);
     }
@@ -470,7 +493,7 @@ __device__ __forceinline__ void closest1_body(const WaveArgs &w, const Lvl &lv, 
         c_closest++; c_fp64 += best[r].nfp64;
         if (best[r].idx >= 0) {
           HitRec *rec = w.hits + hslot[r];
-          hit = finish_hit(a, best[r], src[r], pix[r], qi[r], wt[r], cr[r], cg[r], cb[r], rec, &c_viol, &c_fp64);
+          hit = finish_hit(a, best[r], src[r], pix[r], qi[r], wt[r], cr[r], cg[r], cb[r], rec, &c_viol, &c_fp64) >= 0;
           if (!hit) rec->idx = -1;
         }
         if (a.r.hit_idx) a.r.hit_idx[(size_t)pix[r] * depth + level] = hit ? w.hits[hslot[r]].idx : -1;
@@ -484,7 +507,7 @@ __device__ __forceinline__ void closest1_body(const WaveArgs &w, const Lvl &lv, 
       c_hits += hit;
     }
   }
-  if (a.r.counters) flush_counts(a.r.counters, level, c_closest, c_hits, 0, 0, c_fp64, c_viol, (unsigned long long)a.N);
+  if (a.r.counters) flush_counts(a.r.counters, level, c_closest, c_hits, 0, 0, c_fp64, c_viol, (unsigned long long)a.N, c_cand, c_walks);
 }
 template <bool kSmem, bool kBvh>
 __global__ void __launch_bounds__(kThreads, RT_CLOSEST_CTAS) k_closest1(const WaveArgs w) {
@@ -494,7 +517,7 @@ __global__ void __launch_bounds__(kThreads, RT_CLOSEST_CTAS) k_closest1(const Wa
   const unsigned char *tabs = a.tabs + (size_t)(a.L + 1) * a.tstride;
   if (kSmem) { stage_tables(smem, tabs, a.stage_bytes); tabs = smem + kSmemHeader; }
   RT_PDL_SYNC();
-  closest1_body<kBvh>(w, lvl_of(w), reinterpret_cast<const float4 *>(tabs));
+  closest1_body<kBvh, kSmem && !kBvh>(w, lvl_of(w), reinterpret_cast<const float4 *>(tabs), smem);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -739,6 +762,48 @@ __device__ __forceinline__ void shadow_body(const WaveArgs &w, const Lvl &lv, un
   }
   if (a.r.counters) flush_counts(a.r.counters, 99, 0, 0, c_shadow, c_occ, c_fp64, 0, (unsigned long long)a.N, c_cand, c_walks, c_fall);
 }
+// Level 0, one CTA: the per-tile ray counts become exclusive offsets in tile order, in place, and their sum the number of
+// rays entering level 1.  The queue position of a reflected ray is thus a function of its tile, not of when a warp got
+// to it: a warp of k_closest1 takes 64 rays of a short horizontal strip of consecutive tiles (complex.txt at 1080p: about
+// 10 reflected rays per tile), and the order is the same in every run.  Each thread scans a contiguous run of tiles (whole uint4: tile_ray is allocated to that size); s =
+// 8 words of scratch shared memory.
+__device__ __noinline__ void tile_offsets(unsigned int *tile_ray, int n, unsigned int *rays, unsigned *s) {
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  const int seg = (n + 4 * kThreads - 1) / (4 * kThreads);        // uint4 per thread
+  uint4 *v = reinterpret_cast<uint4 *>(tile_ray) + (size_t)t * seg;
+  const int i0 = t * seg * 4;
+  unsigned sum = 0;
+#pragma unroll 8
+  for (int k = 0; k < seg; k++) {
+    const uint4 c = v[k];
+    const int i = i0 + 4 * k;
+    sum += (i < n ? c.x : 0u) + (i + 1 < n ? c.y : 0u) + (i + 2 < n ? c.z : 0u) + (i + 3 < n ? c.w : 0u);
+  }
+  unsigned incl = sum;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const unsigned y = __shfl_up_sync(kFull, incl, o);
+    if (lane >= o) incl += y;
+  }
+  if (lane == 31) s[warp] = incl;
+  __syncthreads();
+  unsigned run = incl - sum, total = 0;
+  for (int k = 0; k < kWarps; k++) { const unsigned x = s[k]; if (k < warp) run += x; total += x; }
+#pragma unroll 8
+  for (int k = 0; k < seg; k++) {
+    const uint4 c = v[k];
+    const int i = i0 + 4 * k;
+    uint4 o;
+    o.x = run; run += i < n ? c.x : 0u;
+    o.y = run; run += i + 1 < n ? c.y : 0u;
+    o.z = run; run += i + 2 < n ? c.z : 0u;
+    o.w = run; run += i + 3 < n ? c.w : 0u;
+    v[k] = o;
+  }
+  if (t == 0) *rays = total;
+  __syncthreads();
+}
+
 template <int kMode>
 __global__ void __launch_bounds__(kThreads, RT_SHADOW_CTAS) k_shadow(const WaveArgs w) {
   extern __shared__ __align__(128) unsigned char smem[];
@@ -750,6 +815,7 @@ __global__ void __launch_bounds__(kThreads, RT_SHADOW_CTAS) k_shadow(const WaveA
   if (kMode == kTabSmem) { if (a.L > 0) stage_tables(smem, tabs, a.stage_bytes); tabs = smem + kSmemHeader; }
   if (kMode == kTabStream) ring_init(smem);
   RT_PDL_SYNC();
+  if (a.level == 0 && blockIdx.x == 0) tile_offsets(w.tile_ray, a.nwtiles, a.q_out_count, reinterpret_cast<unsigned *>(smem + 64));   // (the header's staging area)
   shadow_body<kMode, false>(w, lvl_of(w), smem, tabs, smem + kSmemHeader + (kMode == kTabBvh ? 0u : ((a.stage_bytes + 127u) & ~127u)));
 }
 
@@ -908,11 +974,18 @@ __global__ void __launch_bounds__(kThreads, RT_DYN_CTAS) k_shadow_dyn(const Wave
 #endif
 constexpr int kShadeUnroll = RT_SHADE_UNROLL;   // 2: both halves of a hit block in one basic block (more loads in flight, more registers)
 __device__ __forceinline__ void prefetch_l1(const void *p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
+// a reflected ray of level 0 at its place in the tile-ordered queue (tile offset + rank); the capacity guard of queue_push
+__device__ __forceinline__ void queue_put(const WaveArgs &w, const Lvl &lv, unsigned pos, const RayRec &rec) {
+  if (pos < w.f.queue_cap) lv.q_out[pos] = rec;
+  else atomicOr(w.f.err, (unsigned)RT_GUARD_RAY_QUEUE);
+}
 
 // The items of this phase cost the same (one hit per lane), so the chunks are dealt out STATICALLY -- warp g of G takes
 // chunks g, g + G, ... -- instead of through an atomic counter: the counter's round trip was a third of this
 // memory-latency-bound kernel's stall samples.  The record of the lane's NEXT hit is prefetched into L1 meanwhile.
-__device__ __forceinline__ void shade_body(const WaveArgs &w, const Lvl &lv) {
+// ordered (level 0 of the wavefront): the reflected rays go to their tile-ordered places (tile_offsets), else they are
+// appended in arrival order (queue_push).
+__device__ __forceinline__ void shade_body(const WaveArgs &w, const Lvl &lv, const bool ordered = false) {
   const FastArgs &a = w.f;
   const unsigned nh = __ldcg(lv.hit_count);
   if (nh == 0u) return;
@@ -944,6 +1017,7 @@ __device__ __forceinline__ void shade_body(const WaveArgs &w, const Lvl &lv) {
       const unsigned pix0 = w.hits[blk * 64u].pix;                  // slot 0 of a block in use always carries its pixel
       const unsigned ty0 = (pix0 / W) & ~(unsigned)(kWTileH - 1), tx0 = (pix0 % W) & ~(unsigned)(kWTileW - 1);
       const bool whole = ty0 + kWTileH <= rows;                      // (W % 16 == 0: every tile is whole in x)
+      const unsigned qbase = ordered ? w.tile_ray[(ty0 / kWTileH) * (unsigned)a.wtiles_x + tx0 / kWTileW] : 0u;
       if (whole) {
 #pragma unroll
         for (int r = 0; r < 2; r++) {                                // the lane's two pixels of the tile, as in k_closest0
@@ -961,6 +1035,7 @@ __device__ __forceinline__ void shade_body(const WaveArgs &w, const Lvl &lv) {
         const bool live = (h & 63u) < nslots && w.hits[h].idx >= 0;
         bool cont = false;
         RayRec rec;
+        unsigned rank = 0;
         if (live) {
           const HitRec hr = w.hits[h];
           unsigned long long occm = hr.pad;
@@ -972,8 +1047,10 @@ __device__ __forceinline__ void shade_body(const WaveArgs &w, const Lvl &lv) {
           c_shadow += (unsigned)L; c_occ += (unsigned)__popcll(occm);
           const unsigned y = hr.pix / W, x = hr.pix - y * W;
           cont = shade_one(w, lv, hr, occm, rec, whole ? s_tile + ((y - ty0) * kWTileW + (x - tx0)) * 3 : nullptr);
+          rank = hit_ray_rank(hr);
         }
-        queue_push(cont, rec, lv.q_out, lv.q_out_count, a.queue_cap, a.err);
+        if (ordered) { if (cont) queue_put(w, lv, qbase + rank, rec); }
+        else queue_push(cont, rec, lv.q_out, lv.q_out_count, a.queue_cap, a.err);
       }
       __syncwarp();
       if (whole && lane < kWTileH * 3) {
@@ -1000,6 +1077,7 @@ __device__ __forceinline__ void shade_body(const WaveArgs &w, const Lvl &lv) {
     const bool live = (h & 63u) < w.hit_n[h >> 6] && w.hits[h].idx >= 0;
     bool cont = false;
     RayRec rec;
+    unsigned qpos = 0;
     if (live) {
       const HitRec hr = w.hits[h];
       unsigned long long occm = hr.pad;
@@ -1010,14 +1088,20 @@ __device__ __forceinline__ void shade_body(const WaveArgs &w, const Lvl &lv) {
       }
       c_shadow += (unsigned)L; c_occ += (unsigned)__popcll(occm);
       cont = shade_one(w, lv, hr, occm, rec);
+      if (ordered && cont) {
+        const unsigned y = hr.pix / (unsigned)a.r.W, x = hr.pix - y * (unsigned)a.r.W;
+        qpos = w.tile_ray[(y / kWTileH) * (unsigned)a.wtiles_x + x / kWTileW] + hit_ray_rank(hr);
+      }
     }
-    queue_push(cont, rec, lv.q_out, lv.q_out_count, a.queue_cap, a.err);
+    if (ordered) { if (cont) queue_put(w, lv, qpos, rec); }
+    else queue_push(cont, rec, lv.q_out, lv.q_out_count, a.queue_cap, a.err);
   }
   if (a.r.counters) flush_counts(a.r.counters, 99, 0, 0, c_shadow, c_occ, 0, 0, (unsigned long long)a.N);
 }
 __global__ void __launch_bounds__(kThreads, RT_SHADE_CTAS) k_shade(const WaveArgs w) {
   RT_PDL_SYNC();
-  shade_body(w, lvl_of(w));
+  const Lvl lv = lvl_of(w);
+  shade_body(w, lv, lv.level == 0);
 }
 
 }  // namespace rtf

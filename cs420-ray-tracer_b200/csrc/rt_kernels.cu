@@ -647,6 +647,7 @@ void rtk_fast_free_work(RtFastWork *w) {
   cudaFree(w->queue[0]); cudaFree(w->queue[1]); cudaFree(w->ctl_base); cudaFree(w->hits); cudaFree(w->occ); cudaFree(w->hit_n); cudaFree(w->cand);
   cudaFree(w->shade_done); w->shade_done = nullptr; w->ctl_base = nullptr; w->last_err = nullptr;
   w->cand = nullptr; w->cand_cap = 0;
+  cudaFree(w->tile_ray); w->tile_ray = nullptr; w->tile_cap = 0;
   if (w->h_fb) { cudaFreeHost(w->h_fb); cudaEventDestroy(w->fb_event); }
   w->h_fb = nullptr; w->fb_pending = 0; w->fb_levels = 0;
   w->queue[0] = w->queue[1] = nullptr; w->ctl = nullptr; w->hits = nullptr; w->occ = nullptr; w->hit_n = nullptr;
@@ -746,6 +747,15 @@ int rtk_launch_fast(const RtRenderArgs &args, const RtFastScene *fs, RtFastWork 
     RTK_TRY(cudaMalloc(&w->cand, npix * sizeof(rtf::Best)));
     w->cand_cap = npix;
   }
+  // per level-0 tile: reflected-ray count, then queue offset (rounded up to whole uint4 segments of the scan, k_shadow)
+  const size_t ntiles = (size_t)((args.W + rtf::kWTileW - 1) / rtf::kWTileW) * ((args.bands.local_rows + rtf::kWTileH - 1) / rtf::kWTileH);
+  const size_t tile_cap = (ntiles + 4 * rtf::kThreads - 1) / (4 * rtf::kThreads) * (4 * rtf::kThreads);
+  if (w->tile_cap < tile_cap) {
+    RTK_TRY(cudaStreamSynchronize(stream));
+    cudaFree(w->tile_ray); w->tile_ray = nullptr; w->tile_cap = 0;
+    RTK_TRY(cudaMalloc(&w->tile_ray, tile_cap * sizeof(unsigned int)));
+    w->tile_cap = tile_cap;
+  }
   // whole-frame kernel: small scenes (every table in shared memory at 2 CTAs/SM), no per-level event marks wanted
   const size_t all_tables = (size_t)(fs->L + 1) * fs->tstride + (size_t)fs->npairs * 32;
   static const int frame_env = getenv("RT_FRAME") ? atoi(getenv("RT_FRAME")) : -1;      // A/B: 0 = wavefront kernels only
@@ -778,7 +788,7 @@ int rtk_launch_fast(const RtRenderArgs &args, const RtFastScene *fs, RtFastWork 
   wa.hits = (rtf::HitRec *)w->hits; wa.hit_cap = (unsigned)hit_cap;   // THIS frame's slot count = the stride of the per-light occlusion rows (the allocation may be
                                                           // larger; with its size as stride a scene with more lights than the one the buffers were sized
                                                           // for would index past occ_bytes)
-  wa.occ = w->occ; wa.hit_n = w->hit_n;
+  wa.occ = w->occ; wa.hit_n = w->hit_n; wa.tile_ray = w->tile_ray;
   wa.occ_bits = fs->L <= 32 && !(getenv("RT_OCC_BYTES") && getenv("RT_OCC_BYTES")[0] == '1');   // (A/B: 1 = occlusion bytes for every scene)
   const size_t pairs_bytes = (size_t)fs->npairs * 32;
   const size_t light_bytes = (size_t)fs->L * fs->tstride;
@@ -881,8 +891,11 @@ int rtk_launch_fast(const RtRenderArgs &args, const RtFastScene *fs, RtFastWork 
     }
     launches++;
     if (level == 0 && marks) RTK_TRY(cudaEventRecord(marks[0], stream));
-    // ---- shadow queries: (light, hit) items
-    if (fs->L > 0) {
+    a.q_out = (rtf::RayRec *)w->queue[level & 1];
+    a.q_out_count = w->ctl + CTL_RAYS + level + 1;
+    // ---- shadow queries: (light, hit) items.  At level 0 also without lights: its CTA 0 turns the per-tile ray counts
+    // into the level-1 queue offsets that k_shade writes to
+    if (fs->L > 0 || level == 0) {
       wa.work_counter = w->ctl + CTL_SHADOW + level;
       a.stage_bytes = (unsigned)light_bytes;
       const size_t smem = light_smem ? staged_smem(a.stage_bytes) : stream_smem;
@@ -897,8 +910,6 @@ int rtk_launch_fast(const RtRenderArgs &args, const RtFastScene *fs, RtFastWork 
     if (level == 0 && marks) RTK_TRY(cudaEventRecord(marks[1], stream));
     // ---- shade + continuation
     wa.work_counter = w->ctl + CTL_SHADE + level;
-    a.q_out = (rtf::RayRec *)w->queue[level & 1];
-    a.q_out_count = w->ctl + CTL_RAYS + level + 1;
     launch(rtf::k_shade, resident_grid(rtf::k_shade, 0, w->num_sms), rtf::kThreads, 0, stream, pdl, wa);
     launches++;
     if (level == 0 && marks) RTK_TRY(cudaEventRecord(marks[2], stream));

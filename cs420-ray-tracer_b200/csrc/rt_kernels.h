@@ -67,6 +67,8 @@ struct RtFastWork {
   size_t cand_cap;
   unsigned char *occ;    // [L][hit_cap] occlusion bytes of the current level
   size_t hit_cap, occ_bytes;
+  unsigned int *tile_ray; // per level-0 tile: its reflected rays, then their first position in the level-1 queue
+  size_t tile_cap;
 };
 int rtk_fast_init(int device);
 // accel: 0 = automatic (LBVH from kBvhAutoSpheres spheres), 1 = table walks only, 2 = LBVH whenever N > 0
