@@ -889,6 +889,12 @@ __device__ __forceinline__ void closest_general_culled(const float4 *__restrict_
                                                        const float (&dy)[NR], const float (&dz)[NR], const bool (&live)[NR], float d64,
                                                        float gS2, float dtmax, const double4 *sph64, const RaySrc (&src)[NR],
                                                        Best (&best)[NR], unsigned short *ids, unsigned &c_cand, unsigned &c_walks) {
+#ifdef RT_NO_GEN_CULL
+  // diagnostics build: the whole table, no bundle walk (unlike RT_NO_CULL, the level-0 and shadow culls stay on); the
+  // culled walk must give the same pixels and the same counters apart from bundle_walks / bundle_candidates
+  closest_general<NR>(pairs, npairs, N, ox, oy, oz, dx, dy, dz, live, d64, gS2, dtmax, sph64, src, best);
+  return;
+#endif
   const Cone cone = warp_cone<NR>(dx, dy, dz, live);
   if (!cone.ok) { closest_general<NR>(pairs, npairs, N, ox, oy, oz, dx, dy, dz, live, d64, gS2, dtmax, sph64, src, best); return; }
   c_walks++;

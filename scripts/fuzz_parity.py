@@ -1,5 +1,9 @@
 """Long-running parity fuzz (not part of the test suite): random adversarial scenes vs the oracle, all kernel families.
-usage: fuzz_parity.py [first_seed] [count] [big|mid]"""
+usage: fuzz_parity.py [first_seed] [count] [big|mid] [--wave-levels]
+
+--wave-levels: the table-mode renders of each seed force rt_set_option wave_levels to one of 1, 2, 3 or 32 (every level a
+wavefront), drawn per seed, each value with a context of its own.  Without it the small frames of this fuzz run their
+reflection levels >= 1 in the tail kernel only."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 for p in (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests"), os.path.join(ROOT, "scripts")):
@@ -7,6 +11,9 @@ for p in (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests"), os.pa
 import numpy as np
 import rtb200, oracle_py
 from test_gpu_parity import _random_scene
+WAVE = "--wave-levels" in sys.argv
+if WAVE:
+    sys.argv.remove("--wave-levels")
 first, count = (int(sys.argv[1]), int(sys.argv[2])) if len(sys.argv) > 2 else (100, 200)
 MID = len(sys.argv) > 3 and sys.argv[3] == "mid"          # 60..300 spheres: tables in shared memory, several fills of a culled walk
 BIG = len(sys.argv) > 3 and sys.argv[3] in ("big", "mid") # 300..4000 spheres: streamed tables (accel=1) and the LBVH
@@ -14,6 +21,11 @@ if BIG:
     import gen_scene
 first0 = first
 rs = {"fast": rtb200.Renderer(0, accel=1 if BIG else None), "bvh": rtb200.Renderer(0, mode="bvh")}
+WAVE_LEVELS = (1, 2, 3, 32)
+rs_wave = {}
+for wl in WAVE_LEVELS if WAVE else ():
+    rs_wave[wl] = rtb200.Renderer(0, accel=1 if BIG else None)
+    rs_wave[wl].set_option("wave_levels", wl)
 bad = 0
 for seed in range(first, first + count):
     g = np.random.default_rng(seed)
@@ -42,7 +54,10 @@ for seed in range(first, first + count):
     if seed % 41 == 0:
         sc = rtb200.Scene(sc.spheres[:0], sc.lights, sc.ambient, sc.camera)      # no spheres
     o = oracle_py.render(sc, W, H, D, want_idx=True)
+    wl = WAVE_LEVELS[int(np.random.default_rng((seed, 1)).integers(len(WAVE_LEVELS)))] if WAVE else 0   # (own stream: the scene's draws stay as they were)
     for m, r in rs.items():
+        if wl and m == "fast":
+            r = rs_wave[wl]
         r.upload(sc)
         first = r.render(W, H, D)[0]                       # (the next frame may pick another wavefront / tail split)
         rgb, hit, mask, st = r.render_debug(W, H, D)
@@ -55,8 +70,8 @@ for seed in range(first, first + count):
             and st.closest_queries == o["counters"]["closest_queries"] and st.occluded == o["counters"]["occluded"]
         if not good:
             bad += 1
-            print("MISMATCH seed %d mode %s: hit %s mask %s rgb %s (%.4f%%, max %d) viol %d" % (
-                seed, m, np.array_equal(hit, o["hit_idx"]), np.array_equal(mask, o["shadow_mask"]), ok_rgb, pct, mx, st.filter_violations))
+            print("MISMATCH seed %d mode %s wave_levels %s: hit %s mask %s rgb %s (%.4f%%, max %d) viol %d" % (
+                seed, m, wl or "auto", np.array_equal(hit, o["hit_idx"]), np.array_equal(mask, o["shadow_mask"]), ok_rgb, pct, mx, st.filter_violations))
             badh = np.argwhere(hit != o["hit_idx"]); badm = np.argwhere(mask != o["shadow_mask"])
             print("   N %d L %d %dx%d d%d; hit mismatches by level %s, mask by level %s, counters gpu (%d %d %d %d) oracle %s" % (
                 sc.nspheres, sc.nlights, W, H, D, np.bincount(badh[:, 2], minlength=D).tolist() if len(badh) else [],
@@ -71,7 +86,7 @@ for seed in range(first, first + count):
             print("   after a second upload of the same scene: hit %s mask %s" % (np.array_equal(hit2, o["hit_idx"]), np.array_equal(mask2, o["shadow_mask"])))
     if seed % 10 == 0:                                   # supersampling and the assembled-frame output mode on the same scene
         import torch
-        r = rs["fast"] if (seed // 10) % 2 == 0 else rs["bvh"]
+        r = (rs_wave[wl] if wl else rs["fast"]) if (seed // 10) % 2 == 0 else rs["bvh"]
         r.upload(sc)
         plain, _ = r.render(W, H, D)
         fr = torch.zeros((H, W, 3), dtype=torch.uint8, device="cuda:0")
@@ -103,5 +118,5 @@ for seed in range(first, first + count):
             bad += 1; print("MISMATCH seed %d: supersampling hit %s rgb %s max %d" % (seed, okk, ok_rgb, mx))
     if (seed - first0 + 1) % 100 == 0:
         print("... %d scenes so far, %d mismatches" % (seed - first0 + 1, bad), flush=True)
-print("fuzz: %d scenes x %d modes, %d mismatches" % (count, len(rs), bad))
+print("fuzz: %d scenes x %d modes%s, %d mismatches" % (count, len(rs), " (tables at wave_levels 1/2/3/32)" if WAVE else "", bad))
 sys.exit(1 if bad else 0)
