@@ -44,6 +44,10 @@ using rtx::d3;
 #endif
 constexpr int kThreads = RT_THREADS;
 constexpr int kWarps = kThreads / 32;
+// work granularity of the wavefront kernels, in units of the grid's warps (measured optimum,
+// profiles/r02_granularity_tunables.txt): two rays / hits per lane from kTwoMult x 64 per warp on; one
+// (chunk, light) shadow item per fetch below kLpMult chunks per warp
+constexpr unsigned kTwoMult = 1, kLpMult = 4;
 constexpr int kWTileW = 16, kWTileH = 4;  // pixels per warp tile (32 lanes x 2 pixels)
 constexpr int kGroupPairs = 4;            // sphere pairs per fast-path group (8 spheres)
 constexpr int kSmemHeader = 2048;         // [0,8) mbarrier, [64, 64+8*192) per-warp RGB staging
@@ -79,8 +83,8 @@ struct FastArgs {
   int tables_in_smem;
   rtb::BvhView bvh;           // large scenes: candidates come from the LBVH instead of a table walk (bvh.cuh)
   int nbig, big[8];           // spheres too large for the LBVH (a ground sphere ...): tested for every ray instead
-  unsigned two_mult, lp_mult; // work-granularity thresholds in units of (warps of the grid): two rays / hits per lane from
-                              // two_mult x 64 per warp on; one (chunk, light) item per fetch below lp_mult chunks per warp
+  unsigned two_mult, lp_mult; // = kTwoMult, kLpMult (launch arguments: folded as constants, they grow the stack frame and
+                              // the spills of k_shadow<kTabBvh>)
   unsigned queue_cap;         // records per ray queue
   unsigned int *err;          // the frame's error word (bounds guards; 0 = clean)
 };

@@ -71,57 +71,25 @@ struct WaveArgs {
   unsigned int *work_counter;      // per-launch chunk counter
   Best *cand;                      // LBVH scenes, level >= 1: per queued ray, the closest-hit candidate k_closest1_dyn found
   unsigned int *work_counter2;     // ... and that kernel's item counter
-  // whole-frame kernel (kernels_frame.cuh): the control words of this frame, those of the next one (zeroed by the kernel
-  // on its way out) and both ray queues; the level-dependent pointers above are derived from these (lvl_at)
-  unsigned int *ctl, *ctl_next;
-  RayRec *queue[2];
-  unsigned int *shade_done;        // per chunk of hits: (chunk, light) items finished so far (self-resetting)
   // per level-0 tile (tile order): the number of its reflected rays (written by k_closest0 for every tile, so never
   // cleared), turned in place into the position of its first ray in the level-1 queue by CTA 0 of the level-0 k_shadow
   unsigned int *tile_ray;
 };
 
-// Control words (u32) of one frame: [0] tile counter, [4] grid-barrier arrivals, [5] error word; per level k <= 33: tail
-// chunk counter, shadow / shade / closest work counters, hits of level k (x64: blocks in use), rays entering level k,
-// shade-done counters of the (chunk, light) items
-enum { CTL_TILE = 0, CTL_BARRIER = 4, CTL_ERR = 5, CTL_TAIL = 8, CTL_SHADOW = 48, CTL_SHADE = 88, CTL_CLOSEST = 128, CTL_HITS = 168, CTL_RAYS = 208,
+// Control words (u32) of one frame: [0] tile counter, [5] error word; per level k <= 33: tail chunk counter, shadow /
+// shade / closest work counters, hits of level k (x64: blocks in use), rays entering level k
+enum { CTL_TILE = 0, CTL_ERR = 5, CTL_TAIL = 8, CTL_SHADOW = 48, CTL_SHADE = 88, CTL_CLOSEST = 128, CTL_HITS = 168, CTL_RAYS = 208,
        CTL_WORDS = 256 };
-
-// The level-dependent part of a launch.  The per-level kernels fill it from their arguments (lvl_of), the whole-frame
-// kernel derives it from the control words (lvl_at).
-struct Lvl {
-  int level;
-  unsigned int *hit_count;                     // 64 x hit blocks in use at this level
-  unsigned int *work_closest, *work_shadow, *work_shade;
-  RayRec *q_in; const unsigned int *q_in_count; // rays entering this level (level >= 1)
-  RayRec *q_out; unsigned int *q_out_count;     // rays leaving it
-};
-__device__ __forceinline__ Lvl lvl_of(const WaveArgs &w) {
-  Lvl v;
-  v.level = w.f.level; v.hit_count = w.hit_count;
-  v.work_closest = v.work_shadow = v.work_shade = w.work_counter;
-  v.q_in = w.f.q_in; v.q_in_count = w.f.q_in_count; v.q_out = w.f.q_out; v.q_out_count = w.f.q_out_count;
-  return v;
-}
-__device__ __forceinline__ Lvl lvl_at(const WaveArgs &w, int level) {
-  Lvl v;
-  v.level = level; v.hit_count = w.ctl + CTL_HITS + level;
-  v.work_closest = level == 0 ? w.ctl + CTL_TILE : w.ctl + CTL_CLOSEST + level;
-  v.work_shadow = w.ctl + CTL_SHADOW + level; v.work_shade = w.ctl + CTL_SHADE + level;
-  v.q_in = w.queue[(level + 1) & 1]; v.q_in_count = w.ctl + CTL_RAYS + level;
-  v.q_out = w.queue[level & 1]; v.q_out_count = w.ctl + CTL_RAYS + level + 1;
-  return v;
-}
 
 // Allocates the block of a work item with (m0, m1) = ballots of its candidate hits; slot[r] = where this
 // lane's hit r goes.  One atomic per work item.
-__device__ __forceinline__ void hit_block(const WaveArgs &w, unsigned int *hit_count, unsigned m0, unsigned m1, unsigned (&slot)[2]) {
+__device__ __forceinline__ void hit_block(const WaveArgs &w, unsigned m0, unsigned m1, unsigned (&slot)[2]) {
   const int lane = threadIdx.x & 31;
   const unsigned n = (unsigned)(__popc(m0) + __popc(m1));
   unsigned base = 0;
   if (n != 0u) {
     if (lane == 0) {
-      base = atomicAdd(hit_count, 64u);
+      base = atomicAdd(w.hit_count, 64u);
       if (base + 64u > w.hit_cap) { atomicOr(w.f.err, (unsigned)RT_GUARD_HIT_BLOCKS); base = 0u; }   // guard: never past the buffer (flagged; block 0 is sacrificed)
       w.hit_n[base >> 6] = n;
     }
@@ -244,12 +212,11 @@ __device__ __forceinline__ unsigned sky_rgb8(float dy) {
   return quant8(c.r) | (quant8(c.g) << 8) | (quant8(c.b) << 16);
 }
 
-// tabs: where table 0 (the camera table) is read from (shared memory when staged); wbase: the per-warp compacted tables;
-// defer_mixed: tiles with hits are stored by the shading pass (tile_path)
+// tabs: where table 0 (the camera table) is read from (shared memory when staged); wbase: the per-warp compacted tables
 template <int kMode>
-__device__ __forceinline__ void closest0_body(const WaveArgs &w, const Lvl &lv, unsigned char *smem, const unsigned char *tabs, unsigned char *wbase,
-                                              const bool defer_mixed) {
+__device__ __forceinline__ void closest0_body(const WaveArgs &w, unsigned char *smem, const unsigned char *tabs, unsigned char *wbase) {
   const FastArgs &a = w.f;
+  const bool defer_mixed = tile_path(a);             // tiles with hits are stored by the shading pass
   const Tab camg = tab_at(a.tabs, a, 0);             // global view (gmin / perm of the streamed mode)
   const Tab cam = tab_at(tabs, a, 0);
   const WarpBuf wb = warp_buf(wbase);                                                                                // kTabSmem / kTabBvh
@@ -264,11 +231,11 @@ __device__ __forceinline__ void closest0_body(const WaveArgs &w, const Lvl &lv, 
   for (;;) {
     int tile;
     if (kMode == kTabStream) {
-      const int ct = cta_fetch(lv.work_closest, smem);
+      const int ct = cta_fetch(a.tile_counter, smem);
       if (ct * kWarps >= a.nwtiles) break;
       tile = ct * kWarps + warp;
     } else {
-      tile = warp_fetch(lv.work_closest);
+      tile = warp_fetch(a.tile_counter);
       if (tile >= a.nwtiles) break;
     }
     const bool tile_ok = tile < a.nwtiles;
@@ -353,7 +320,7 @@ __device__ __forceinline__ void closest0_body(const WaveArgs &w, const Lvl &lv, 
     }
     unsigned hslot[2];
     const unsigned hm0 = __ballot_sync(kFull, live[0] && best[0].idx >= 0), hm1 = __ballot_sync(kFull, live[1] && best[1].idx >= 0);
-    hit_block(w, lv.hit_count, hm0, hm1, hslot);
+    hit_block(w, hm0, hm1, hslot);
     // a whole tile with a hit block: the shading pass stores it (tile_path)
     const bool deferred = defer_mixed && (hm0 | hm1) != 0u && tx0 + kWTileW <= W && ty0 + kWTileH <= rows;
     bool cont[2];                                    // the hit's path continues (shade_one's test): a level-1 ray
@@ -427,9 +394,7 @@ __global__ void __launch_bounds__(kThreads, RT_CLOSEST0_CTAS) k_closest0(const W
   if (kMode == kTabSmem) { stage_tables(smem, a.tabs, a.stage_bytes); tabs = smem + kSmemHeader; }
   if (kMode == kTabStream) ring_init(smem);
   RT_PDL_SYNC();
-  Lvl lv = lvl_of(w);
-  lv.work_closest = a.tile_counter;
-  closest0_body<kMode>(w, lv, smem, tabs, smem + kSmemHeader + (kMode == kTabBvh ? 0u : ((a.stage_bytes + 127u) & ~127u)), tile_path(a));
+  closest0_body<kMode>(w, smem, tabs, smem + kSmemHeader + (kMode == kTabBvh ? 0u : ((a.stage_bytes + 127u) & ~127u)));
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -437,20 +402,20 @@ __global__ void __launch_bounds__(kThreads, RT_CLOSEST0_CTAS) k_closest0(const W
 // gen: the general table (shared memory when staged); kCull (gen staged): bundle-culled walk, survivors listed in the
 // header's per-warp staging area (unused in this kernel: kGenIds 16-bit slots of its 192 bytes)
 template <bool kBvh, bool kCull = false>
-__device__ __forceinline__ void closest1_body(const WaveArgs &w, const Lvl &lv, const float4 *gen, unsigned char *smem = nullptr) {
+__device__ __forceinline__ void closest1_body(const WaveArgs &w, const float4 *gen, unsigned char *smem) {
   const FastArgs &a = w.f;
-  const unsigned nq = __ldcg(lv.q_in_count);
+  const unsigned nq = __ldcg(a.q_in_count);
   if (nq == 0u) return;
-  const int lane = threadIdx.x & 31, depth = a.r.max_depth, level = lv.level;
+  const int lane = threadIdx.x & 31, depth = a.r.max_depth, level = a.level;
   unsigned c_closest = 0, c_hits = 0, c_fp64 = 0, c_viol = 0, c_cand = 0, c_walks = 0;
-  const RayRec *qin = lv.q_in;
+  const RayRec *qin = a.q_in;
   static_assert(kGenIds * 2 <= kWTileH * kWTileW * 3, "survivor list in the header's per-warp staging area");
   unsigned short *ids = kCull ? reinterpret_cast<unsigned short *>(smem + 64 + (threadIdx.x >> 5) * (kWTileH * kWTileW * 3)) : nullptr;
   // few rays (deep levels): one ray per lane, so that twice as many warps share the work
   const bool two = nq >= gridDim.x * (unsigned)kWarps * 64u * a.two_mult;
   const unsigned per = two ? 64u : 32u;
   for (;;) {
-    const int chunk = warp_fetch(lv.work_closest);
+    const int chunk = warp_fetch(w.work_counter);
     if ((unsigned)chunk * per >= nq) break;
     bool live[2];
     unsigned qi[2], pix[2];
@@ -470,14 +435,10 @@ __device__ __forceinline__ void closest1_body(const WaveArgs &w, const Lvl &lv, 
     Best best[2];
     best_init(best[0]); best_init(best[1]);
     const RaySrc src[2] = {{nullptr, nullptr, 0, 0, qin + qi[0]}, {nullptr, nullptr, 0, 0, qin + qi[1]}};
-    if (kBvh && w.cand) {                            // the traversal already ran (k_closest1_dyn): pick up its result
+    if (kBvh) {                                      // the traversal already ran (k_closest1_dyn): pick up its result
 #pragma unroll
       for (int r = 0; r < 2; r++)
         if (live[r]) best[r] = w.cand[qi[r]];
-    } else if (kBvh) {
-#pragma unroll 1
-      for (int r = 0; r < 2; r++)
-        if (live[r]) best[r] = bvh_closest_general(a, gen, ox[r], oy[r], oz[r], dx[r], dy[r], dz[r], src[r]);
     } else if (kCull) {
       closest_general_culled<2>(gen, a.npairs, a.N, ox, oy, oz, dx, dy, dz, live, a.d64, a.gS2, a.g_dtmax, a.r.sph64, src, best, ids,
                                 c_cand, c_walks);
@@ -485,7 +446,7 @@ __device__ __forceinline__ void closest1_body(const WaveArgs &w, const Lvl &lv, 
       closest_general<2>(gen, a.npairs, a.N, ox, oy, oz, dx, dy, dz, live, a.d64, a.gS2, a.g_dtmax, a.r.sph64, src, best);
     }
     unsigned hslot[2];
-    hit_block(w, lv.hit_count, __ballot_sync(kFull, live[0] && best[0].idx >= 0), __ballot_sync(kFull, live[1] && best[1].idx >= 0), hslot);
+    hit_block(w, __ballot_sync(kFull, live[0] && best[0].idx >= 0), __ballot_sync(kFull, live[1] && best[1].idx >= 0), hslot);
 #pragma unroll
     for (int r = 0; r < 2; r++) {
       bool hit = false;
@@ -517,7 +478,7 @@ __global__ void __launch_bounds__(kThreads, RT_CLOSEST_CTAS) k_closest1(const Wa
   const unsigned char *tabs = a.tabs + (size_t)(a.L + 1) * a.tstride;
   if (kSmem) { stage_tables(smem, tabs, a.stage_bytes); tabs = smem + kSmemHeader; }
   RT_PDL_SYNC();
-  closest1_body<kBvh, kSmem && !kBvh>(w, lvl_of(w), reinterpret_cast<const float4 *>(tabs), smem);
+  closest1_body<kBvh, kSmem && !kBvh>(w, reinterpret_cast<const float4 *>(tabs), smem);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -526,10 +487,10 @@ __global__ void __launch_bounds__(kThreads, RT_CLOSEST_CTAS) k_closest1(const Wa
 // or the path continues: returns true and *rec is the exact FP64 reflected ray for the next level's queue.
 // stage != nullptr: a final pixel is not written to the frame but quantised into stage[0..2] (the caller emits whole
 // 16-byte row segments of its tile), *is_final tells which it was.
-__device__ __forceinline__ bool shade_one(const WaveArgs &w, const Lvl &lv, const HitRec &hr, unsigned long long occm, RayRec &rec,
+__device__ __forceinline__ bool shade_one(const WaveArgs &w, const int level, const HitRec &hr, unsigned long long occm, RayRec &rec,
                                           unsigned char *stage = nullptr) {
   const FastArgs &a = w.f;
-  const int L = a.L, level = lv.level;
+  const int L = a.L;
   const float4 m = __ldg(&a.r.mat[hr.idx]);
   const float2 mx = __ldg(&a.r.matx[hr.idx]);
   float sr = g_frame.ambient[0] * m.x, sg = g_frame.ambient[1] * m.y, sb = g_frame.ambient[2] * m.z;
@@ -549,7 +510,7 @@ __device__ __forceinline__ bool shade_one(const WaveArgs &w, const Lvl &lv, cons
       // the normal from the exact hit point (src/main.cpp:35,45-48)
       d3 din;
       if (cam) din = rtx::mk(hit_d0x(hr), hit_d0y(hr), hit_d0z(hr));
-      else { const RayRec &q = lv.q_in[hr.src]; din = rtx::mk(q.dx, q.dy, q.dz); }
+      else { const RayRec &q = a.q_in[hr.src]; din = rtx::mk(q.dx, q.dy, q.dz); }
       const double4 s = ld_sph64(&a.r.sph64[hr.idx]);
       const d3 p = rtx::mk(hr.px, hr.py, hr.pz);
       reflected_ray_from_center(din, p, rtx::mk(s.x, s.y, s.z), &rec);
@@ -576,16 +537,12 @@ __device__ __forceinline__ bool shade_one(const WaveArgs &w, const Lvl &lv, cons
 // that sphere's exit distance, which is shorter than the distance to any light outside that sphere
 // (flag bit 30 of Tab::inv, set on the host): occluded, no table walk needed.
 // tabs: where the L light tables are read from (shared memory when staged); wbase: the per-warp compacted tables.
-// kFuse (whole-frame kernel): the warp that knows the last occlusion bit of a chunk of hits also SHADES it -- directly
-// from its registers when it ran all lights of the chunk itself, or, when the (chunk, light) items of a chunk are spread
-// over several warps, as the last of them to arrive (one arrival counter per chunk; the occlusion bytes of the others
-// are read back through L2) -- so the 80-byte hit records are not streamed from HBM a second time by a shade kernel.
-template <int kMode, bool kFuse>
-__device__ __forceinline__ void shadow_body(const WaveArgs &w, const Lvl &lv, unsigned char *smem, const unsigned char *tabs, unsigned char *wbase) {
+template <int kMode>
+__device__ __forceinline__ void shadow_body(const WaveArgs &w, unsigned char *smem, const unsigned char *tabs, unsigned char *wbase) {
   const FastArgs &a = w.f;
   const unsigned char *gtabs = a.tabs + a.tstride;
-  const unsigned nh = __ldcg(lv.hit_count);
-  if (nh == 0u || (a.L == 0 && !kFuse)) return;
+  const unsigned nh = __ldcg(w.hit_count);
+  if (nh == 0u || a.L == 0) return;
   const WarpBuf wb = warp_buf(wbase);                                                                                // kTabSmem / kTabBvh
   const BundleBuf bb = bundle_buf(smem + kSmemHeader + kWarps * kWarpBufBytes);                                      // kTabBvh only
   unsigned ring_phase = 0;
@@ -597,22 +554,19 @@ __device__ __forceinline__ void shadow_body(const WaveArgs &w, const Lvl &lv, un
   // as many, L times shorter items, so the warps of the machine share them evenly
   const bool lightpar = kMode != kTabStream && a.L > 1 && nchunks < a.lp_mult * gridDim.x * (unsigned)kWarps;
   const unsigned nitems = lightpar ? nchunks * (unsigned)a.L : nchunks;
-  unsigned c_fp64 = 0, c_cand = 0, c_walks = 0, c_fall = 0, c_shadow = 0, c_occ = 0;
+  unsigned c_fp64 = 0, c_cand = 0, c_walks = 0, c_fall = 0;
   for (;;) {
     unsigned chunk;
     if (kMode == kTabStream) {
-      const unsigned cc = (unsigned)cta_fetch(lv.work_shadow, smem);
+      const unsigned cc = (unsigned)cta_fetch(w.work_counter, smem);
       if (cc * kWarps >= nchunks) break;
       chunk = cc * kWarps + warp;
     } else {
-      chunk = (unsigned)warp_fetch(lv.work_shadow);
+      chunk = (unsigned)warp_fetch(w.work_counter);
       if (chunk >= nitems) break;
     }
     int l_beg = 0, l_end = a.L;
     if (lightpar) { l_beg = (int)(chunk % (unsigned)a.L); l_end = l_beg + 1; chunk /= (unsigned)a.L; }
-    // occlusion bits of this lane's two hits (fused shading: up to 64 lights; record bits: <= 32, half the registers)
-    typedef unsigned long long OccT;
-    OccT occm[2] = {0, 0};                             // (fused shading only)
     const unsigned h0 = two ? chunk * 64u + 2u * lane : chunk * 32u + lane;
     const unsigned hend = (h0 & ~63u) + (h0 < nh ? w.hit_n[h0 >> 6] : 0u);   // end of the block's live slots
     bool have[2];
@@ -711,11 +665,6 @@ __device__ __forceinline__ void shadow_body(const WaveArgs &w, const Lvl &lv, un
         occ[0] = q.occ[0]; occ[1] = q.occ[1];
       }
       c_fp64 += (unsigned)n64;
-      if (kFuse && !lightpar) {                        // this warp runs every light of the chunk: the bits stay in registers
-        if (occ[0] || shortcut[0]) occm[0] |= (OccT)1 << l;
-        if (occ[1] || shortcut[1]) occm[1] |= (OccT)1 << l;
-        continue;
-      }
       if (w.occ_bits) {                                // one fire-and-forget RED.OR per OCCLUDED (hit, light) into the hit record
         if (have[0] && (occ[0] || shortcut[0])) atomicOr(&w.hits[h0].pad, 1u << l);
         if (have[1] && (occ[1] || shortcut[1])) atomicOr(&w.hits[h0 + 1].pad, 1u << l);
@@ -727,40 +676,8 @@ __device__ __forceinline__ void shadow_body(const WaveArgs &w, const Lvl &lv, un
       if (have[1]) *reinterpret_cast<unsigned short *>(o) = (unsigned short)(o0 | o1);
       else if (have[0]) o[0] = (unsigned char)o0;
     }
-    if (!kFuse) continue;
-    if (lightpar) {
-      // the last of the chunk's L items to arrive shades it; its own bytes are in L2 after the fence, the others' are
-      // read back with L1-bypassing loads
-      __threadfence();
-      __syncwarp();
-      unsigned last = 0u;
-      if (lane == 0) {
-        last = atomicAdd(&w.shade_done[chunk], 1u) == (unsigned)a.L - 1u ? 1u : 0u;
-        if (last) w.shade_done[chunk] = 0u;            // ready for the next level / frame
-      }
-      if (!__shfl_sync(kFull, last, 0)) continue;
-      __threadfence();
-#pragma unroll
-      for (int r = 0; r < 2; r++)
-        if (have[r]) {
-          if (w.occ_bits) occm[r] = __ldcg(&w.hits[h0 + r].pad);
-          else
-            for (int l = 0; l < a.L; l++)
-              if (__ldcg(w.occ + (size_t)l * w.hit_cap + h0 + r)) occm[r] |= (OccT)1 << l;
-        }
-    }
-#pragma unroll
-    for (int r = 0; r < 2; r++) {
-      bool cont = false;
-      RayRec rec;
-      if (have[r]) {
-        c_shadow += (unsigned)a.L; c_occ += (unsigned)__popcll((unsigned long long)occm[r]);
-        cont = shade_one(w, lv, w.hits[h0 + r], (unsigned long long)occm[r], rec);
-      }
-      queue_push(cont, rec, lv.q_out, lv.q_out_count, a.queue_cap, a.err);
-    }
   }
-  if (a.r.counters) flush_counts(a.r.counters, 99, 0, 0, c_shadow, c_occ, c_fp64, 0, (unsigned long long)a.N, c_cand, c_walks, c_fall);
+  if (a.r.counters) flush_counts(a.r.counters, 99, 0, 0, 0, 0, c_fp64, 0, (unsigned long long)a.N, c_cand, c_walks, c_fall);
 }
 // Level 0, one CTA: the per-tile ray counts become exclusive offsets in tile order, in place, and their sum the number of
 // rays entering level 1.  The queue position of a reflected ray is thus a function of its tile, not of when a warp got
@@ -816,7 +733,7 @@ __global__ void __launch_bounds__(kThreads, RT_SHADOW_CTAS) k_shadow(const WaveA
   if (kMode == kTabStream) ring_init(smem);
   RT_PDL_SYNC();
   if (a.level == 0 && blockIdx.x == 0) tile_offsets(w.tile_ray, a.nwtiles, a.q_out_count, reinterpret_cast<unsigned *>(smem + 64));   // (the header's staging area)
-  shadow_body<kMode, false>(w, lvl_of(w), smem, tabs, smem + kSmemHeader + (kMode == kTabBvh ? 0u : ((a.stage_bytes + 127u) & ~127u)));
+  shadow_body<kMode>(w, smem, tabs, smem + kSmemHeader + (kMode == kTabBvh ? 0u : ((a.stage_bytes + 127u) & ~127u)));
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -975,19 +892,21 @@ __global__ void __launch_bounds__(kThreads, RT_DYN_CTAS) k_shadow_dyn(const Wave
 constexpr int kShadeUnroll = RT_SHADE_UNROLL;   // 2: both halves of a hit block in one basic block (more loads in flight, more registers)
 __device__ __forceinline__ void prefetch_l1(const void *p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
 // a reflected ray of level 0 at its place in the tile-ordered queue (tile offset + rank); the capacity guard of queue_push
-__device__ __forceinline__ void queue_put(const WaveArgs &w, const Lvl &lv, unsigned pos, const RayRec &rec) {
-  if (pos < w.f.queue_cap) lv.q_out[pos] = rec;
+__device__ __forceinline__ void queue_put(const WaveArgs &w, unsigned pos, const RayRec &rec) {
+  if (pos < w.f.queue_cap) w.f.q_out[pos] = rec;
   else atomicOr(w.f.err, (unsigned)RT_GUARD_RAY_QUEUE);
 }
 
 // The items of this phase cost the same (one hit per lane), so the chunks are dealt out STATICALLY -- warp g of G takes
 // chunks g, g + G, ... -- instead of through an atomic counter: the counter's round trip was a third of this
 // memory-latency-bound kernel's stall samples.  The record of the lane's NEXT hit is prefetched into L1 meanwhile.
-// ordered (level 0 of the wavefront): the reflected rays go to their tile-ordered places (tile_offsets), else they are
-// appended in arrival order (queue_push).
-__device__ __forceinline__ void shade_body(const WaveArgs &w, const Lvl &lv, const bool ordered = false) {
+// Level 0: the reflected rays go to their tile-ordered places (tile_offsets); levels >= 1 append them in arrival order
+// (queue_push).
+__device__ __forceinline__ void shade_body(const WaveArgs &w) {
   const FastArgs &a = w.f;
-  const unsigned nh = __ldcg(lv.hit_count);
+  const int level = a.level;
+  const bool ordered = level == 0;
+  const unsigned nh = __ldcg(w.hit_count);
   if (nh == 0u) return;
   const int lane = threadIdx.x & 31, L = a.L;
   unsigned c_shadow = 0, c_occ = 0;
@@ -996,7 +915,7 @@ __device__ __forceinline__ void shade_body(const WaveArgs &w, const Lvl &lv, con
   // block and stores the whole tile as twelve 16-byte row segments: every pixel starts as the sky colour of its camera
   // ray (what k_closest0 would have written), the finished hits overwrite theirs in shared memory, the hits whose path
   // continues are overwritten later by the level that finishes them.  k_closest0 leaves such tiles alone (tile_path).
-  if (lv.level == 0 && tile_path(a)) {
+  if (ordered && tile_path(a)) {
     __shared__ __align__(16) unsigned char s_tiles[kWarps][kWTileH * kWTileW * 3];
     unsigned char *s_tile = s_tiles[threadIdx.x >> 5];
     const unsigned W = (unsigned)a.r.W, rows = (unsigned)a.r.bands.local_rows;
@@ -1017,7 +936,7 @@ __device__ __forceinline__ void shade_body(const WaveArgs &w, const Lvl &lv, con
       const unsigned pix0 = w.hits[blk * 64u].pix;                  // slot 0 of a block in use always carries its pixel
       const unsigned ty0 = (pix0 / W) & ~(unsigned)(kWTileH - 1), tx0 = (pix0 % W) & ~(unsigned)(kWTileW - 1);
       const bool whole = ty0 + kWTileH <= rows;                      // (W % 16 == 0: every tile is whole in x)
-      const unsigned qbase = ordered ? w.tile_ray[(ty0 / kWTileH) * (unsigned)a.wtiles_x + tx0 / kWTileW] : 0u;
+      const unsigned qbase = w.tile_ray[(ty0 / kWTileH) * (unsigned)a.wtiles_x + tx0 / kWTileW];
       if (whole) {
 #pragma unroll
         for (int r = 0; r < 2; r++) {                                // the lane's two pixels of the tile, as in k_closest0
@@ -1046,11 +965,10 @@ __device__ __forceinline__ void shade_body(const WaveArgs &w, const Lvl &lv, con
           }
           c_shadow += (unsigned)L; c_occ += (unsigned)__popcll(occm);
           const unsigned y = hr.pix / W, x = hr.pix - y * W;
-          cont = shade_one(w, lv, hr, occm, rec, whole ? s_tile + ((y - ty0) * kWTileW + (x - tx0)) * 3 : nullptr);
+          cont = shade_one(w, level, hr, occm, rec, whole ? s_tile + ((y - ty0) * kWTileW + (x - tx0)) * 3 : nullptr);
           rank = hit_ray_rank(hr);
         }
-        if (ordered) { if (cont) queue_put(w, lv, qbase + rank, rec); }
-        else queue_push(cont, rec, lv.q_out, lv.q_out_count, a.queue_cap, a.err);
+        if (cont) queue_put(w, qbase + rank, rec);
       }
       __syncwarp();
       if (whole && lane < kWTileH * 3) {
@@ -1087,21 +1005,20 @@ __device__ __forceinline__ void shade_body(const WaveArgs &w, const Lvl &lv, con
           if (w.occ[(size_t)l * w.hit_cap + h]) occm |= 1ull << l;
       }
       c_shadow += (unsigned)L; c_occ += (unsigned)__popcll(occm);
-      cont = shade_one(w, lv, hr, occm, rec);
+      cont = shade_one(w, level, hr, occm, rec);
       if (ordered && cont) {
         const unsigned y = hr.pix / (unsigned)a.r.W, x = hr.pix - y * (unsigned)a.r.W;
         qpos = w.tile_ray[(y / kWTileH) * (unsigned)a.wtiles_x + x / kWTileW] + hit_ray_rank(hr);
       }
     }
-    if (ordered) { if (cont) queue_put(w, lv, qpos, rec); }
-    else queue_push(cont, rec, lv.q_out, lv.q_out_count, a.queue_cap, a.err);
+    if (ordered) { if (cont) queue_put(w, qpos, rec); }
+    else queue_push(cont, rec, a.q_out, a.q_out_count, a.queue_cap, a.err);
   }
   if (a.r.counters) flush_counts(a.r.counters, 99, 0, 0, c_shadow, c_occ, 0, 0, (unsigned long long)a.N);
 }
 __global__ void __launch_bounds__(kThreads, RT_SHADE_CTAS) k_shade(const WaveArgs w) {
   RT_PDL_SYNC();
-  const Lvl lv = lvl_of(w);
-  shade_body(w, lv, lv.level == 0);
+  shade_body(w);
 }
 
 }  // namespace rtf

@@ -118,7 +118,6 @@ extern "C" int rt_create(int device, rt_ctx **out) {
   memset(&c->fast, 0, sizeof(c->fast));
   memset(&c->work, 0, sizeof(c->work));
   c->work.num_sms = prop.multiProcessorCount;
-  c->work.frame_kernel = -1;
   // (a failure below must not leak the half-built context: rt_destroy copes with null members)
   cudaError_t ce = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking);
   if (ce == cudaSuccess) ce = cudaEventCreate(&c->ev0);
@@ -178,7 +177,6 @@ extern "C" int rt_set_option(rt_ctx *c, const char *key, long long value) {
   if (!strcmp(key, "counters")) { c->counters_on = value != 0; return RT_OK; }
   if (!strcmp(key, "antialias")) { c->antialias = value != 0; return RT_OK; }
   if (!strcmp(key, "level_timing")) { c->level_timing = value != 0; return RT_OK; }
-  if (!strcmp(key, "frame_kernel")) { c->work.frame_kernel = value < 0 ? -1 : (value != 0); return RT_OK; }
   if (!strcmp(key, "accel")) {
     if (value < 0 || value > 2) return rt_fail(RT_ERR_ARG, "rt_set_option: accel must be 0 (auto), 1 (tables) or 2 (LBVH)");
     c->accel = (int)value;
@@ -388,7 +386,7 @@ static int collect_stats(rt_ctx *c, rt_stats *stats) {
     const int er = rtk_fast_last_error(&c->work, &word);
     if (er != 0) return rt_fail(RT_ERR_CUDA, std::string("render: reading the error word failed: ") + cudaGetErrorString((cudaError_t)-er));
     if (word != 0)
-      return rt_fail(RT_ERR_STATE, "render: device-side guard tripped (bit 0: hit-block buffer, bit 1: ray queue, else: grid barrier timeout): word " +
+      return rt_fail(RT_ERR_STATE, "render: device-side guard tripped (bit 0: hit-block buffer, bit 1: ray queue): word " +
                                        std::to_string(word));
   }
   if (c->pend_counters) {

@@ -3,8 +3,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <map>
 #include <mutex>
@@ -18,7 +16,6 @@ __constant__ RtFrameConst g_frame;
 #include "kernels_exact.cuh"
 #include "kernels_fast.cuh"
 #include "kernels_wave.cuh"
-#include "kernels_frame.cuh"
 
 cudaError_t rtk_set_frame_const(const RtFrameConst *host_const, cudaStream_t stream) {
   return cudaMemcpyToSymbolAsync(g_frame, host_const, sizeof(RtFrameConst), 0, cudaMemcpyHostToDevice, stream);
@@ -37,7 +34,7 @@ int rtk_launch_exact(const RtRenderArgs &args, cudaStream_t stream) {
 namespace {
 
 constexpr size_t kMaxSmemTables = 90 * 1024;    // stage a kernel's tables in shared memory up to this size (2 CTAs/SM stay resident)
-constexpr int kCtlWords = rtf::CTL_WORDS;        // device control words per frame, layout: enum CTL_* (kernels_wave.cuh); two sets (see rtk_launch_fast)
+constexpr int kCtlWords = rtf::CTL_WORDS;        // device control words per frame, layout: enum CTL_* (kernels_wave.cuh)
 
 inline float float_up(double x) {               // smallest float >= x
   float f = (float)x;
@@ -64,8 +61,6 @@ int rtk_fast_init(int) {
   RTK_TRY(cudaFuncSetAttribute(rtf::k_shadow<rtf::kTabStream>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
   RTK_TRY(cudaFuncSetAttribute(rtf::k_shadow<rtf::kTabBvh>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
   RTK_TRY(cudaFuncSetAttribute(rtf::k_closest0<rtf::kTabBvh>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-  RTK_TRY(cudaFuncSetAttribute(rtf::k_frame<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-  RTK_TRY(cudaFuncSetAttribute(rtf::k_frame<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
   RTK_TRY(cudaFuncSetAttribute(rtb::k_bvh_sort, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((16 * rtb::kSortThreads + 32) * sizeof(unsigned))));
   return 0;
 }
@@ -374,7 +369,7 @@ int rtk_fast_build_scene(RtFastScene *fs, const double *sph, int N, const RtFram
   // spheres on they are written by a kernel from the raw rows (k_build_lookup) instead of staged on the host.
   const bool lookup_only = N > 0 && (accel == 2 || (accel == 0 && N >= kBvhAutoSpheres));
   constexpr int kDeviceBuildSpheres = 2048;
-  const bool device_build = lookup_only && N >= kDeviceBuildSpheres && !(getenv("RT_HOST_BUILD") && getenv("RT_HOST_BUILD")[0] == '1');
+  const bool device_build = lookup_only && N >= kDeviceBuildSpheres;
   fs->lookup_only = lookup_only; fs->device_build = device_build;
   // byte layout of one shared-origin table
   const unsigned pairs_bytes = (unsigned)npairs * 32u;
@@ -635,7 +630,7 @@ void rtk_fast_free_scene(RtFastScene *fs, int release_tables) {
 }
 
 // The error word of the last frame launched (call after the stream has been synchronised): bounds guards of the hit /
-// ray queues, grid-barrier timeout of the whole-frame kernel.  0 = clean.
+// ray queues.  0 = clean.
 int rtk_fast_last_error(const RtFastWork *w, unsigned int *word) {
   *word = 0;
   if (!w->last_err) return 0;
@@ -644,8 +639,8 @@ int rtk_fast_last_error(const RtFastWork *w, unsigned int *word) {
 }
 
 void rtk_fast_free_work(RtFastWork *w) {
-  cudaFree(w->queue[0]); cudaFree(w->queue[1]); cudaFree(w->ctl_base); cudaFree(w->hits); cudaFree(w->occ); cudaFree(w->hit_n); cudaFree(w->cand);
-  cudaFree(w->shade_done); w->shade_done = nullptr; w->ctl_base = nullptr; w->last_err = nullptr;
+  cudaFree(w->queue[0]); cudaFree(w->queue[1]); cudaFree(w->ctl); cudaFree(w->hits); cudaFree(w->occ); cudaFree(w->hit_n); cudaFree(w->cand);
+  w->last_err = nullptr;
   w->cand = nullptr; w->cand_cap = 0;
   cudaFree(w->tile_ray); w->tile_ray = nullptr; w->tile_cap = 0;
   if (w->h_fb) { cudaFreeHost(w->h_fb); cudaEventDestroy(w->fb_event); }
@@ -669,9 +664,7 @@ int resident_grid(K kernel, size_t smem, int num_sms, int threads = rtf::kThread
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, threads, smem) != cudaSuccess || nb < 1) nb = 1;
     it = cache.emplace(key, nb).first;
   }
-  // RT_GRID_DIV (experiments): a fraction of the resident grid, so that the kernels of two contexts can share the SMs
-  static const int grid_div = getenv("RT_GRID_DIV") ? std::max(1, atoi(getenv("RT_GRID_DIV"))) : 1;
-  return std::max(1, it->second * num_sms / grid_div);
+  return std::max(1, it->second * num_sms);
 }
 // Launch with programmatic dependent launch (PDL): the grid may start while the previous kernel of the stream is
 // still draining, run its prologue (table staging) and then block in griddepcontrol.wait (RT_PDL_SYNC in the kernels)
@@ -679,19 +672,14 @@ int resident_grid(K kernel, size_t smem, int num_sms, int threads = rtf::kThread
 // The first failing launch of a frame is remembered (g_launch_err, thread local) and reported by rtk_launch_fast.
 thread_local cudaError_t g_launch_err = cudaSuccess;
 template <typename K, typename A>
-void launch(K kernel, int grid, int block, size_t smem, cudaStream_t stream, bool pdl, const A &arg, bool cooperative = false) {
+void launch(K kernel, int grid, int block, size_t smem, cudaStream_t stream, bool pdl, const A &arg) {
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)block); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
   cudaLaunchAttribute at[1];
-  if (cooperative) {            // every CTA of the grid co-resident (the whole-frame kernel has grid-wide barriers)
-    at[0].id = cudaLaunchAttributeCooperative;
-    at[0].val.cooperative = 1;
-  } else {
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-  }
-  cfg.attrs = at; cfg.numAttrs = (pdl || cooperative) ? 1u : 0u;
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = at; cfg.numAttrs = pdl ? 1u : 0u;
   const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, arg);
   if (e != cudaSuccess && g_launch_err == cudaSuccess) g_launch_err = e;
 }
@@ -707,30 +695,18 @@ using rtf::CTL_TILE; using rtf::CTL_TAIL; using rtf::CTL_SHADOW; using rtf::CTL_
 int rtk_launch_fast(const RtRenderArgs &args, const RtFastScene *fs, RtFastWork *w, cudaStream_t stream,
                     const cudaEvent_t *marks) {
   const size_t npix = (size_t)args.W * args.bands.local_rows;
-  static const unsigned two_mult = getenv("RT_TWO_MULT") ? (unsigned)atoi(getenv("RT_TWO_MULT")) : 1u;   // tunables (A/B on the GPU)
-  static const unsigned lp_mult = getenv("RT_LP_MULT") ? (unsigned)atoi(getenv("RT_LP_MULT")) : 4u;
-  if (!w->ctl_base) {
-    // two sets of control words: the whole-frame kernel zeroes the set of the NEXT frame on its way out, so no memset
-    // precedes it in steady state
-    RTK_TRY(cudaMalloc(&w->ctl_base, 2 * kCtlWords * sizeof(unsigned int)));
-    RTK_TRY(cudaMemsetAsync(w->ctl_base, 0, 2 * kCtlWords * sizeof(unsigned int), stream));
-    w->ctl_clean[0] = w->ctl_clean[1] = 1; w->ctl_cur = 0;
-  }
-  w->ctl = w->ctl_base + (size_t)w->ctl_cur * kCtlWords;
+  if (!w->ctl) RTK_TRY(cudaMalloc(&w->ctl, kCtlWords * sizeof(unsigned int)));
   // blocked hit queue: one 64-slot block per 16x4 tile (level 0: tiles x 64 >= pixels) or per 64 queued rays (level >= 1:
   // at most pixels / 64 + 1 blocks).  With few rays (fewer than one per lane of the resident grid) k_closest1 takes 32 rays
   // per block instead: fewer than grid x 8 warps x 2 blocks; the slack term covers the largest resident grid (4 CTAs/SM).
   const size_t hit_cap = ((size_t)((args.W + rtf::kWTileW - 1) / rtf::kWTileW) * ((args.bands.local_rows + rtf::kWTileH - 1) / rtf::kWTileH) + 2) * 64 +
-                         (size_t)w->num_sms * 4 * rtf::kWarps * 128 * (size_t)two_mult;
+                         (size_t)w->num_sms * 4 * rtf::kWarps * 128 * (size_t)rtf::kTwoMult;
   if (w->hit_cap < hit_cap || w->occ_bytes < hit_cap * (size_t)(fs->L > 0 ? fs->L : 1) || (args.max_depth > 1 && w->queue_cap < npix)) {
     RTK_TRY(cudaStreamSynchronize(stream));
     cudaFree(w->queue[0]); cudaFree(w->queue[1]); cudaFree(w->hits); cudaFree(w->occ); cudaFree(w->hit_n);
     w->queue[0] = w->queue[1] = nullptr; w->hits = nullptr; w->occ = nullptr; w->hit_n = nullptr; w->queue_cap = w->hit_cap = w->occ_bytes = 0;
     RTK_TRY(cudaMalloc(&w->hits, hit_cap * sizeof(rtf::HitRec)));
     RTK_TRY(cudaMalloc(&w->hit_n, (hit_cap / 64) * sizeof(unsigned int)));
-    cudaFree(w->shade_done); w->shade_done = nullptr;
-    RTK_TRY(cudaMalloc(&w->shade_done, (hit_cap / 32 + 1) * sizeof(unsigned int)));
-    RTK_TRY(cudaMemsetAsync(w->shade_done, 0, (hit_cap / 32 + 1) * sizeof(unsigned int), stream));
     w->occ_bytes = hit_cap * (size_t)(fs->L > 0 ? fs->L : 1);
     RTK_TRY(cudaMalloc(&w->occ, w->occ_bytes));
     w->hit_cap = hit_cap;
@@ -756,16 +732,7 @@ int rtk_launch_fast(const RtRenderArgs &args, const RtFastScene *fs, RtFastWork 
     RTK_TRY(cudaMalloc(&w->tile_ray, tile_cap * sizeof(unsigned int)));
     w->tile_cap = tile_cap;
   }
-  // whole-frame kernel: small scenes (every table in shared memory at 2 CTAs/SM), no per-level event marks wanted
-  const size_t all_tables = (size_t)(fs->L + 1) * fs->tstride + (size_t)fs->npairs * 32;
-  static const int frame_env = getenv("RT_FRAME") ? atoi(getenv("RT_FRAME")) : -1;      // A/B: 0 = wavefront kernels only
-  const int frame_opt = w->frame_kernel >= 0 ? w->frame_kernel : frame_env;
-  // (measured: the per-level kernels win -- each has its own register budget and occupancy -- so the whole-frame kernel
-  // runs only on request: rt_set_option frame_kernel 1 / RT_FRAME=1; DESIGN.md 5d)
-  const bool use_frame = frame_opt > 0 && !fs->bvh_nodes && all_tables <= kMaxSmemTables && marks == nullptr && args.max_depth > 0 &&
-                         w->wave_levels <= 0;
-  if (!use_frame || !w->ctl_clean[w->ctl_cur]) RTK_TRY(cudaMemsetAsync(w->ctl, 0, kCtlWords * sizeof(unsigned int), stream));
-  w->ctl_clean[w->ctl_cur] = 0;
+  RTK_TRY(cudaMemsetAsync(w->ctl, 0, kCtlWords * sizeof(unsigned int), stream));
   if (args.max_depth <= 0 && !args.fb && !args.out_remap) RTK_TRY(cudaMemsetAsync(args.rgb, 0, npix * 3, stream));   // src/main.cpp:17-18: black (other output modes: the caller clears)
 
   g_launch_err = cudaSuccess;
@@ -782,14 +749,14 @@ int rtk_launch_fast(const RtRenderArgs &args, const RtFastScene *fs, RtFastWork 
   a.wtiles_x = (args.W + rtf::kWTileW - 1) / rtf::kWTileW;
   a.nwtiles = a.wtiles_x * ((args.bands.local_rows + rtf::kWTileH - 1) / rtf::kWTileH);
   a.tile_counter = w->ctl + CTL_TILE;
-  a.two_mult = two_mult; a.lp_mult = lp_mult;
+  a.two_mult = rtf::kTwoMult; a.lp_mult = rtf::kLpMult;
   a.queue_cap = (unsigned)w->queue_cap; a.err = w->ctl + rtf::CTL_ERR;
   w->last_err = a.err;
   wa.hits = (rtf::HitRec *)w->hits; wa.hit_cap = (unsigned)hit_cap;   // THIS frame's slot count = the stride of the per-light occlusion rows (the allocation may be
                                                           // larger; with its size as stride a scene with more lights than the one the buffers were sized
                                                           // for would index past occ_bytes)
   wa.occ = w->occ; wa.hit_n = w->hit_n; wa.tile_ray = w->tile_ray;
-  wa.occ_bits = fs->L <= 32 && !(getenv("RT_OCC_BYTES") && getenv("RT_OCC_BYTES")[0] == '1');   // (A/B: 1 = occlusion bytes for every scene)
+  wa.occ_bits = fs->L <= 32;
   const size_t pairs_bytes = (size_t)fs->npairs * 32;
   const size_t light_bytes = (size_t)fs->L * fs->tstride;
   // per kernel: its tables are staged whole when they fit, else streamed (shared-origin tables) or read through L1/L2 (general table)
@@ -803,10 +770,8 @@ int rtk_launch_fast(const RtRenderArgs &args, const RtFastScene *fs, RtFastWork 
   // larger tables are streamed through a two-stage ring of TMA tiles (kernels_wave.cuh, kTabStream)
   const size_t stream_smem = rtf::kSmemHeader + 2 * (size_t)rtf::kTileBytes;
   int launches = 0;
-  // event records between the kernels (stats) break the launch adjacency PDL needs; RT_NO_PDL=1 turns it off (A/B)
-  static const bool pdl_env = !(getenv("RT_NO_PDL") && getenv("RT_NO_PDL")[0] == '1');
-  const bool pdl = pdl_env && marks == nullptr;
-  static const bool bvh_dyn = !(getenv("RT_BVH_DYN") && getenv("RT_BVH_DYN")[0] == '0');   // A/B: 0 = warp-synchronous LBVH shadow kernel
+  // event records between the kernels (stats) break the launch adjacency PDL needs
+  const bool pdl = marks == nullptr;
 
   // levels below wave_levels run as phase-separated wavefront kernels; the (few) rays left after that are
   // followed to termination by one fused launch
@@ -832,33 +797,6 @@ int rtk_launch_fast(const RtRenderArgs &args, const RtFastScene *fs, RtFastWork 
     }
     if (w->fb_levels > 0 && w->fb_key == fb_key) wave_levels = w->fb_levels;
   }
-  if (use_frame) {
-    wa.ctl = w->ctl; wa.ctl_next = w->ctl_base + (size_t)(w->ctl_cur ^ 1) * kCtlWords;
-    wa.queue[0] = (rtf::RayRec *)w->queue[0]; wa.queue[1] = (rtf::RayRec *)w->queue[1];
-    wa.shade_done = w->shade_done;
-    a.level = 0;
-    a.stage_bytes = (unsigned)all_tables;
-    const size_t smem = staged_smem(all_tables);
-    static const bool fuse = !(getenv("RT_FUSE") && getenv("RT_FUSE")[0] == '0');      // A/B: 0 = shading as its own phase
-    int g = fuse ? resident_grid(rtf::k_frame<true>, smem, w->num_sms) : resident_grid(rtf::k_frame<false>, smem, w->num_sms);
-    const int cta_tiles = (a.nwtiles + rtf::kWarps - 1) / rtf::kWarps;
-    if (g > cta_tiles) g = cta_tiles;                  // (a tiny frame: fewer CTAs than fit is still co-resident)
-    if (fuse) launch(rtf::k_frame<true>, g, rtf::kThreads, smem, stream, false, wa, true);
-    else launch(rtf::k_frame<false>, g, rtf::kThreads, smem, stream, false, wa, true);
-    if (getenv("RT_FRAME_TRACE")) {                    // diagnostics: phase boundaries seen by CTA 0 (ns timer)
-      unsigned int tr[14];
-      cudaStreamSynchronize(stream);
-      cudaMemcpy(tr, w->ctl + 242, sizeof(tr), cudaMemcpyDeviceToHost);
-      fprintf(stderr, "k_frame phases (us):");
-      for (int k = 1; k < 14 && tr[k]; k++) fprintf(stderr, " %.1f", (tr[k] - tr[k - 1]) * 1e-3);
-      fprintf(stderr, "\n");
-    }
-    w->ctl_clean[w->ctl_cur ^ 1] = 1;                  // zeroed by the kernel
-    w->ctl_cur ^= 1;
-    cudaError_t e = cudaGetLastError();
-    if (g_launch_err != cudaSuccess) e = g_launch_err;
-    return e == cudaSuccess ? 1 : -(int)e;
-  }
   for (int level = 0; level < args.max_depth && level < wave_levels; level++) {
     a.level = level;
     wa.hit_count = w->ctl + CTL_HITS + level;
@@ -877,13 +815,11 @@ int rtk_launch_fast(const RtRenderArgs &args, const RtFastScene *fs, RtFastWork 
       a.stage_bytes = (unsigned)pairs_bytes;
       const size_t smem = rtf::kSmemHeader + (gen_smem ? a.stage_bytes : 0);
       if (bvh) {
-        wa.cand = nullptr;
-        if (bvh_dyn && w->cand && w->cand_cap >= npix) {                    // incoherent rays: traversal with dynamic ray fetch, then the coherent finish
-          wa.cand = (rtf::Best *)w->cand;
-          wa.work_counter2 = w->ctl + CTL_TAIL + level;     // (the tail's counters are unused in LBVH scenes)
-          launch(rtf::k_closest1_dyn, resident_grid(rtf::k_closest1_dyn, 0, w->num_sms), rtf::kThreads, 0, stream, pdl, wa);
-          launches++;
-        }
+        // incoherent rays: traversal with dynamic ray fetch, then the coherent finish
+        wa.cand = (rtf::Best *)w->cand;
+        wa.work_counter2 = w->ctl + CTL_TAIL + level;       // (the tail's counters are unused in LBVH scenes)
+        launch(rtf::k_closest1_dyn, resident_grid(rtf::k_closest1_dyn, 0, w->num_sms), rtf::kThreads, 0, stream, pdl, wa);
+        launches++;
         launch(rtf::k_closest1<false, true>, resident_grid(rtf::k_closest1<false, true>, rtf::kSmemHeader, w->num_sms), rtf::kThreads, rtf::kSmemHeader, stream, pdl, wa);
       }
       else if (gen_smem) launch(rtf::k_closest1<true, false>, resident_grid(rtf::k_closest1<true, false>, smem, w->num_sms), rtf::kThreads, smem, stream, pdl, wa);
@@ -901,7 +837,7 @@ int rtk_launch_fast(const RtRenderArgs &args, const RtFastScene *fs, RtFastWork 
       const size_t smem = light_smem ? staged_smem(a.stage_bytes) : stream_smem;
       // camera-ray hits are coherent: the warp-synchronous kernel wins at level 0 (4.3 vs 5.9 ms on config 4); from level 1 on
       // the rays are not, and the dynamic-fetch kernel does (levels >= 1 of config 5: 57.6 -> 38 ms)
-      if (bvh && bvh_dyn && level > 0) launch(rtf::k_shadow_dyn, resident_grid(rtf::k_shadow_dyn, 0, w->num_sms), rtf::kThreads, 0, stream, pdl, wa);
+      if (bvh && level > 0) launch(rtf::k_shadow_dyn, resident_grid(rtf::k_shadow_dyn, 0, w->num_sms), rtf::kThreads, 0, stream, pdl, wa);
       else if (bvh) launch(rtf::k_shadow<rtf::kTabBvh>, resident_grid(rtf::k_shadow<rtf::kTabBvh>, bvh_smem(), w->num_sms), rtf::kThreads, bvh_smem(), stream, pdl, wa);
       else if (light_smem) launch(rtf::k_shadow<rtf::kTabSmem>, resident_grid(rtf::k_shadow<rtf::kTabSmem>, smem, w->num_sms), rtf::kThreads, smem, stream, pdl, wa);
       else launch(rtf::k_shadow<rtf::kTabStream>, resident_grid(rtf::k_shadow<rtf::kTabStream>, smem, w->num_sms), rtf::kThreads, smem, stream, pdl, wa);

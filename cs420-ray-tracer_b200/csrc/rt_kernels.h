@@ -56,11 +56,8 @@ struct RtFastWork {
   unsigned long long fb_key, fb_pending_key;
   void *queue[2];        // reflected-ray records, ping-pong between levels
   size_t queue_cap;      // records per queue
-  unsigned int *ctl;     // device control words of the current frame: tile counter, per-level chunk counters, queue counts
-  unsigned int *ctl_base; int ctl_cur, ctl_clean[2];   // two sets; clean = known to be all zero
-  unsigned int *shade_done;   // whole-frame kernel: per chunk of hits, (chunk, light) shadow items finished (self-resetting)
-  unsigned int *last_err; // device: error word of the last frame launched (bounds guards, barrier timeout)
-  int frame_kernel;      // -1 automatic (whole-frame kernel when every table fits in shared memory), 0 never, 1 = as automatic
+  unsigned int *ctl;     // device control words (zeroed before every frame): tile counter, per-level chunk counters, queue counts
+  unsigned int *last_err; // device: error word of the last frame launched (bounds guards)
   void *hits;            // HitRec queue of the current level (kernels_wave.cuh), 64-slot blocks
   unsigned int *hit_n;   // hits per block
   void *cand;            // LBVH scenes: closest-hit candidate per queued ray (k_closest1_dyn -> k_closest1)

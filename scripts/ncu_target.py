@@ -1,5 +1,5 @@
 """Target for ncu captures: a few production frames (no stats) of one configuration.
-usage: ncu_target.py scene W H D frames [frame_kernel]"""
+usage: ncu_target.py scene W H D frames"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
@@ -13,8 +13,6 @@ if name.startswith("synth"):
 else:
     sc = rtb200.load_scene(os.path.join(os.path.dirname(__file__), "..", "tests", "golden", "scenes", name + ".txt"))
 r = rtb200.Renderer(0)
-if len(sys.argv) > 6:
-    r.set_option("frame_kernel", int(sys.argv[6]))
 r.upload(sc)
 out = np.empty((H, W, 3), dtype=np.uint8)
 for _ in range(frames):

@@ -17,13 +17,9 @@ for label, scene, kw, sizes in [("tables/smem", cx, {}, [(97, 61, 4), (160, 90, 
             rgb, hit, mask, st = r.render_debug(W, H, D)
             print(label, W, H, D, "rays", st.closest_queries + st.shadow_queries, "viol", st.filter_violations)
         if kw.get("mode") != "exact":
-            # production launch sequence (no stats: programmatic dependent launch) and the whole-frame cooperative kernel
+            # production launch sequence (no stats: programmatic dependent launch)
             r.render(160, 90, 5, want_stats=False)
             r.render(160, 90, 5, want_stats=False)
-            r.set_option("frame_kernel", 1)
-            r.render_debug(97, 61, 4)
-            r.render(160, 90, 5, want_stats=False)
-            r.set_option("frame_kernel", 0)
             r.set_option("antialias", 1)
             r.render(50, 30, 3)
             r.set_option("antialias", 0)

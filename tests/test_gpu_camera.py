@@ -173,16 +173,6 @@ def test_supersampling(rt, scenes):
 
 
 @gpu
-def test_whole_frame_kernel_option(rt, scenes):
-    sc = scenes["complex"]
-    # (the whole-frame kernel gathers the rays of its tail into warps in the order they arrive, so the counters of its
-    # table walks vary from run to run even for one upload: here only the ray counts, which the frame defines, are
-    # compared; the camera table itself is covered by the tests above)
-    follow(rt, sc, orbit(sc.camera, 4, turn=1.0)[1:], opts={"frame_kernel": 1},
-           counters=("closest_queries", "hits", "shadow_queries", "occluded", "sphere_tests"))
-
-
-@gpu
 @pytest.mark.parametrize("mode", ["fast", "bvh"])
 def test_bands_frame_and_tiles(rt, scenes, mode):
     import torch

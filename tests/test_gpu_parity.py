@@ -324,6 +324,8 @@ def test_errors(rt, renderers, scenes):
         r.render(0, 16, 2)
     with pytest.raises(rt.RtError):
         r.render(16, 16, 33)
+    with pytest.raises(rt.RtError, match="unknown key"):
+        r.set_option("frame_kernel", 1)
     r.close()
 
 
@@ -451,21 +453,6 @@ def test_upload_waits_for_renders_on_caller_streams(rt, oracle, scenes):
         for n in gold:
             ok, pct, mx = rt.compare_rgb(gold[n], bufs[n][:H * W * 3].cpu().numpy().reshape(H, W, 3), 0.5)
             assert ok and mx <= 2, (n, pct, mx)
-
-
-@pytest.mark.parametrize("name,W,H,D", [("complex", 320, 180, 5), ("simple", 200, 120, 10), ("medium", 97, 61, 3)])
-def test_whole_frame_kernel_option(rt, oracle, scenes, name, W, H, D):
-    """rt_set_option frame_kernel 1: the whole frame as ONE cooperative persistent kernel (grid barriers between the
-    phases, shading fused into the shadow phase; csrc/kernels_frame.cuh).  Slower than the per-level kernels on a B200
-    (DESIGN.md 5d) and therefore off by default, but kept bit-exact: same indices, masks, counters and pixels."""
-    with rt.Renderer(0) as r:
-        r.set_option("frame_kernel", 1)
-        for _ in range(3):
-            check(rt, oracle, r, scenes[name], W, H, D)
-        a, _ = r.render(W, H, D)
-        r.set_option("frame_kernel", 0)
-        b, _ = r.render(W, H, D)
-        assert np.array_equal(a, b)
 
 
 @pytest.mark.parametrize("mode", ["fast", "bvh"])
