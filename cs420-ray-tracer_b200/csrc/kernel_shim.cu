@@ -14,7 +14,8 @@
 // What differs, by necessity: the reference's caller hands the scene over as FP32 device structs, so the scene this
 // shim renders is the FP32-rounded one (exactly what the reference's own kernel sees); it is rendered with the serial
 // renderer's semantics by librt_b200 (rt_render_tile).  The sphere array and the camera are read back from the device
-// once per (pointer, count) and cached; call kernel_shim_invalidate() after changing them in place.  Errors cannot be
+// once per (sphere pointer, camera pointer, sphere count, light count) and cached; call kernel_shim_invalidate() after
+// changing them in place.  Errors cannot be
 // returned through a void function: like the reference's CUDA_CHECK (include/gpu_shared.h:14-22) they are printed and
 // the process exits.
 #include <cuda_runtime.h>
@@ -40,7 +41,7 @@ rt_ctx *g_ctx = nullptr;
 std::vector<double> g_lights;            // L x 7, file column order
 double g_ambient[3] = {0, 0, 0};
 const void *g_spheres_ptr = nullptr, *g_camera_ptr = nullptr;
-int g_nspheres = -1;
+int g_nspheres = -1, g_nlights = -1;
 bool g_dirty = true;
 
 [[noreturn]] void die(const char *what) {
@@ -82,7 +83,8 @@ extern "C" void launch_gpu_kernel(float3 *d_framebuffer, ShimSphere *d_spheres, 
     die_cuda("cudaGetDevice", cudaGetDevice(&dev));
     if (rt_create(dev, &g_ctx) != RT_OK) die("rt_create");
   }
-  if (g_dirty || d_spheres != g_spheres_ptr || camera != g_camera_ptr || num_spheres != g_nspheres) {
+  if (g_dirty || d_spheres != g_spheres_ptr || camera != g_camera_ptr || num_spheres != g_nspheres ||
+      num_lights != g_nlights) {
     // (blocking copies: once per scene; they also order this read behind the caller's own uploads)
     std::vector<ShimSphere> hs((size_t)(num_spheres > 0 ? num_spheres : 0));
     if (num_spheres > 0) die_cuda("read spheres", cudaMemcpy(hs.data(), d_spheres, hs.size() * sizeof(ShimSphere), cudaMemcpyDeviceToHost));
@@ -101,7 +103,7 @@ extern "C" void launch_gpu_kernel(float3 *d_framebuffer, ShimSphere *d_spheres, 
     const double look[3] = {pos[0] + (double)cam.forward.x, pos[1] + (double)cam.forward.y, pos[2] + (double)cam.forward.z};
     if (rt_upload_scene(g_ctx, sph.data(), (int)hs.size(), g_lights.data(), L, g_ambient, pos, look, (double)cam.fov) != RT_OK)
       die("rt_upload_scene");
-    g_spheres_ptr = d_spheres; g_camera_ptr = camera; g_nspheres = num_spheres; g_dirty = false;
+    g_spheres_ptr = d_spheres; g_camera_ptr = camera; g_nspheres = num_spheres; g_nlights = num_lights; g_dirty = false;
   }
   if (rt_render_tile(g_ctx, image_width, image_height, max_depth, tile_x, tile_y, tile_width, tile_height,
                      reinterpret_cast<float *>(d_framebuffer), (void *)stream) != RT_OK)
