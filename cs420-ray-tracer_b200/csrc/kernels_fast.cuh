@@ -19,7 +19,7 @@
 // origin (camera / one light) and form a narrow bundle.  The warp bounds them by a cone, tests every
 // sphere of the table against that cone ONCE (one sphere per lane, warp ballot), compacts the
 // survivors into a per-warp shared-memory table and runs the per-ray tests over that table only:
-// a handful of spheres instead of all N.  The cone test is conservative (see cull_round).
+// a handful of spheres instead of all N.  The cone test is conservative (margins: see Cone).
 //
 // What is FP32 and what is FP64:  every ray/sphere TEST is 4 packed-FP32 FMAs per sphere pair
 // (FFMA2; shared origin) or 10 (general origin).  The tests are conservative (filter_math.cuh);
@@ -39,10 +39,7 @@ namespace rtf {
 
 using rtx::d3;
 
-#ifndef RT_THREADS
-#define RT_THREADS 256
-#endif
-constexpr int kThreads = RT_THREADS;
+constexpr int kThreads = 256;               // per CTA of the wavefront kernels (DESIGN §5d: 128-thread CTAs were slower)
 constexpr int kWarps = kThreads / 32;
 // work granularity of the wavefront kernels, in units of the grid's warps (measured optimum,
 // profiles/r02_granularity_tunables.txt): two rays / hits per lane from kTwoMult x 64 per warp on; one
@@ -366,11 +363,8 @@ __device__ __forceinline__ bool shared_origin_roots(float ocx, float ocy, float 
 
 // ---- slow paths: one flagged sphere PAIR for ONE ray.  The FP32 bracketing is inline (a call would
 // spill the caller's registers to local memory around it); only the FP64 deciders are out of line.
-#ifndef RT_SLOW
-#define RT_SLOW __forceinline__
-#endif
-__device__ RT_SLOW Best slow_closest_shared(Best b, const float4 *pairs, const int *perm, int pi, float dx, float dy, float dz,
-                                                 float d64, const double4 *sph64, RaySrc src) {
+__device__ __forceinline__ Best slow_closest_shared(Best b, const float4 *pairs, const int *perm, int pi, float dx, float dy, float dz,
+                                                         float d64, const double4 *sph64, RaySrc src) {
   const float4 A = pairs[2 * pi], B = pairs[2 * pi + 1];
 #pragma unroll 1
   for (int h = 0; h < 2; h++) {
@@ -390,8 +384,8 @@ __device__ RT_SLOW Best slow_closest_shared(Best b, const float4 *pairs, const i
 }
 
 // returns bit 0 = an occluder was found in this pair, bits 1.. = FP64 evaluations spent
-__device__ RT_SLOW int slow_shadow(const float4 *pairs, const int *perm, int pi, float dx, float dy, float dz, float so, float m,
-                                        int self, float cosl, const double *p3, int light, float d64, const double4 *sph64) {
+__device__ __forceinline__ int slow_shadow(const float4 *pairs, const int *perm, int pi, float dx, float dy, float dz, float so, float m,
+                                                int self, float cosl, const double *p3, int light, float d64, const double4 *sph64) {
   const float so_lo = so - m, so_hi = so + m, e_lo = -kEps - m, e_hi = -kEps + m;
   const float4 A = pairs[2 * pi], B = pairs[2 * pi + 1];
   int n64 = 0, found = 0;
@@ -417,8 +411,8 @@ __device__ RT_SLOW int slow_shadow(const float4 *pairs, const int *perm, int pi,
   return found | (n64 << 1);
 }
 
-__device__ RT_SLOW Best slow_closest_general(Best b, const float4 *pairs, int pi, int N, float ox, float oy, float oz, float dx,
-                                                  float dy, float dz, float d64, float gS2, const double4 *sph64, RaySrc src) {
+__device__ __forceinline__ Best slow_closest_general(Best b, const float4 *pairs, int pi, int N, float ox, float oy, float oz, float dx,
+                                                          float dy, float dz, float d64, float gS2, const double4 *sph64, RaySrc src) {
   const float sS = __fsqrt_ru(gS2);
   const float4 A = pairs[2 * pi], B = pairs[2 * pi + 1];
 #pragma unroll 1
@@ -612,34 +606,11 @@ __device__ __forceinline__ WarpBuf warp_buf(unsigned char *base) {
   return b;
 }
 
-// One culling round: lane l looks at slot base + l of table T.  Survivors (ballot order = table order,
-// so the compacted table stays sorted) are copied to positions ncand.. of the warp's table.  `wcut`:
-// spheres whose group lies beyond it are dropped as well.  Returns the survivors' ballot mask.
-__device__ __forceinline__ unsigned cull_round(const Tab &T, int base, int nslots, const Cone &c, float wcut, const WarpBuf &wb,
-                                               int ncand) {
-  const int lane = threadIdx.x & 31, slot = base + lane;
-  bool keep = false;
-  if (slot < nslots) {
-    const float4 u = T.cullA[slot];
-    const float sA = T.cullB[slot];
-    const float dotv = fabsf(fmaf(u.z, c.az, fmaf(u.y, c.ay, u.x * c.ax)));
-    keep = !(dotv < fmaf(c.cth, u.w, -fmaf(c.sth, sA, 2e-5f))) && !(T.gmin[slot >> 3] > wcut);
-  }
-  const unsigned mk = __ballot_sync(kFull, keep);
-  if (keep) {
-    const int rank = ncand + __popc(mk & ((1u << lane) - 1u));
-    const float *src = reinterpret_cast<const float *>(T.pairs) + (slot >> 1) * 8 + (slot & 1);
-    float *dst = reinterpret_cast<float *>(wb.pairs) + (rank >> 1) * 8 + (rank & 1);
-    dst[0] = src[0]; dst[2] = src[2]; dst[4] = src[4]; dst[6] = src[6];
-    wb.perm[rank] = T.perm[slot];
-    if ((rank & 7) == 0) wb.gmin[rank >> 3] = T.gmin[slot >> 3];    // lower bound of this and every later key
-  }
-  return mk;
-}
-// Two culling rounds at once: lane l looks at slots base + l AND base + 32 + l.  The two cone tests are independent
-// dependency chains in one basic block (the single round is bound by its own chain: shared-memory load -> 5 dependent FMAs
-// -> compare -> ballot -> compaction), and half the loop iterations, ballots and cut-off checks remain.  Same test, same
-// survivor order (table order), so the compacted table is the one two single rounds would have produced.
+// Two culling rounds at once: lane l looks at slots base + l AND base + 32 + l of table T.  Survivors (ballot order = table
+// order, so the compacted table stays sorted) are copied to positions ncand.. of the warp's table.  `wcut`: spheres whose
+// group lies beyond it are dropped as well.  mk0 / mk1: the survivors' ballot masks of the two rounds.  The two cone tests
+// are independent dependency chains in one basic block (a single round is bound by its own chain: shared-memory load -> 5
+// dependent FMAs -> compare -> ballot -> compaction), and half the loop iterations, ballots and cut-off checks remain.
 __device__ __forceinline__ void cull_round2(const Tab &T, int base, int nslots, const Cone &c, float wcut, const WarpBuf &wb, int ncand,
                                             unsigned &mk0, unsigned &mk1) {
   const int lane = threadIdx.x & 31, s0 = base + lane, s1 = s0 + 32;
@@ -1001,8 +972,7 @@ __device__ __forceinline__ bool shadow_range(ShadowQ<NR> &q, const float4 *__res
                                              int pend, int light, const float (&dx)[NR], const float (&dy)[NR], const float (&dz)[NR],
                                              const float (&so)[NR], const int (&self)[NR], const float (&cosl)[NR],
                                              const double *const (&p64)[NR], float d64, const double4 *sph64, int &n_fp64,
-                                             const bool coop = false, const unsigned char *mixed_tabs = nullptr, unsigned tstride = 0u,
-                                             unsigned long long *prof = nullptr) {
+                                             const bool coop = false, const unsigned char *mixed_tabs = nullptr, unsigned tstride = 0u) {
   float2 dx2[NR], dy2[NR], dz2[NR];
 #pragma unroll
   for (int r = 0; r < NR; r++) { dx2[r] = make_float2(dx[r], dx[r]); dy2[r] = make_float2(dy[r], dy[r]); dz2[r] = make_float2(dz[r], dz[r]); }
@@ -1012,8 +982,6 @@ __device__ __forceinline__ bool shadow_range(ShadowQ<NR> &q, const float4 *__res
     else if (gmin[p0 / kGroupPairs] > q.wcut) return false;
     const int np = min(kChunkPairs, pend - p0);
     unsigned h[NR], f[NR], any = 0u;
-    long long pt0 = 0;
-    if (prof) pt0 = clock64();
     if (NR == 1 && kMixed && coop) h[0] = ~coop_chunk_mixed(mixed_tabs, tstride, light, p0, np, dx[0], dy[0], dz[0], q.open[0]);
     else if (NR == 1 && coop) h[0] = ~coop_chunk_shared(pairs, p0, np, dx[0], dy[0], dz[0], q.open[0]);
     else chunk_test_shared<NR>(pairs, p0, np, dx2, dy2, dz2, h);
@@ -1030,13 +998,11 @@ __device__ __forceinline__ bool shadow_range(ShadowQ<NR> &q, const float4 *__res
       }
       any |= f[r];
     }
-    if (prof) { const long long t = clock64(); prof[0] += (unsigned long long)(t - pt0); prof[3]++; pt0 = t; }
     if (__any_sync(kFull, any != 0u)) {
 #pragma unroll
       for (int r = 0; r < NR; r++) {
         unsigned fr = f[r];
         while (__any_sync(kFull, fr != 0u)) {
-          if (prof) prof[2]++;
           if (fr != 0u) {
             const int bit = 31 - __clz(fr);
             const int pi = p0 + np - 1 - bit;
@@ -1055,7 +1021,6 @@ __device__ __forceinline__ bool shadow_range(ShadowQ<NR> &q, const float4 *__res
 #pragma unroll
       for (int r = 0; r < NR; r++) c = fmaxf(c, q.open[r] ? q.cut[r] : -3.0e38f);   // decided rays stop holding the warp
       q.wcut = wmaxf(c);
-      if (prof) prof[1] += (unsigned long long)(clock64() - pt0);
       if (q.wcut < -1.0e38f) return false;
     }
   }
@@ -1078,8 +1043,7 @@ __device__ __forceinline__ void shadow_light(const Tab T, int npairs, int light,
 // its lanes: ceil(hits x L / 32) walks instead of L walks with the lanes of the missed rays idle).  Same chunk tests, same
 // slow paths and deciders per (ray, sphere) as shadow_light, so the same booleans.
 __device__ __forceinline__ bool shadow_mixed(const unsigned char *tabs, const FastArgs &a, int light, float dx, float dy, float dz, float so,
-                                             bool want, int self, float cosl, const double *p64, int &n_fp64, const bool coop,
-                                             unsigned long long *prof = nullptr) {
+                                             bool want, int self, float cosl, const double *p64, int &n_fp64, const bool coop) {
   const Tab T = tab_at(tabs, a, light);
   const float dxa[1] = {dx}, dya[1] = {dy}, dza[1] = {dz}, soa[1] = {so}, cosla[1] = {cosl};
   const bool wanta[1] = {want};
@@ -1088,7 +1052,7 @@ __device__ __forceinline__ bool shadow_mixed(const unsigned char *tabs, const Fa
   ShadowQ<1> q;
   shadow_begin<1>(q, T.inv, soa, wanta, selfa, cosla);
   shadow_range<1, true>(q, T.pairs, T.gmin, T.perm, 0, a.npairs, light, dxa, dya, dza, soa, selfa, cosla, pa, a.d64, a.r.sph64, n_fp64, coop, tabs,
-                        a.tstride, prof);
+                        a.tstride);
   return q.occ[0];
 }
 
@@ -1203,7 +1167,7 @@ __device__ __forceinline__ bool bvh_shadow(const FastArgs &a, const Tab T, float
 }
 
 // ---------------------------------------------------------------------------------------------
-// BUNDLE TRAVERSAL of the LBVH: bundle culling (see cull_round) for scenes too large for a table scan.  The warp's
+// BUNDLE TRAVERSAL of the LBVH: bundle culling (margins: see Cone) for scenes too large for a table scan.  The warp's
 // ray bundle descends the hierarchy BREADTH FIRST with the lanes working on 32 frontier nodes at a time: a child
 // survives when the interval-arithmetic slab test (bundle_slab) cannot exclude that some ray of the bundle touches its
 // (inflated) box within the distance cutoff.  Surviving leaves name candidate spheres; these are gathered into the warp's compacted table
@@ -1412,27 +1376,10 @@ __device__ __forceinline__ void flush_counters(const FastArgs &a, Counters &c, i
 // warp's chain: closest hit -> exact t / geometry -> shadow queries -> Phong -> reflect.  The shadow
 // queries were two thirds of that chain when every light was walked in turn with the lanes of the missed
 // rays idle; now the self-shadow shortcut settles the back-facing half and the rest is packed 32 per walk
-// (profiles/r02_tail_phase_trace.txt; -DRT_TAIL_TRACE builds the phase stamps in).
-#ifndef RT_TAIL_THREADS
-#define RT_TAIL_THREADS 128
-#endif
-#ifndef RT_TAIL_CTAS
-#define RT_TAIL_CTAS 3
-#endif
-constexpr int kTailThreads = RT_TAIL_THREADS;
-#ifdef RT_TAIL_TRACE
-// diagnostics build only (scripts/probe_tail_trace.py): per warp (first chunk), per level, SM-clock stamps of the phases
-constexpr int kTraceWarps = 4096, kTraceLevels = 6, kTraceStamps = 12;
-__device__ unsigned long long g_tail_trace[kTraceWarps * kTraceLevels * kTraceStamps];
-#define RT_TT(k, extra) do { const unsigned long long x_ = (unsigned long long)(extra);   /* (warp-wide: ballots inside) */ \
-    if (tt_on && lane == 0 && level - a.level < kTraceLevels) g_tail_trace[(tt_warp * kTraceLevels + (level - a.level)) * kTraceStamps + (k)] = (unsigned long long)clock64() | (x_ << 48); } while (0)
-#define RT_TG(k) do { if (tt_on && lane == 0 && level - a.level < kTraceLevels) { unsigned long long t_; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t_)); g_tail_trace[(tt_warp * kTraceLevels + (level - a.level)) * kTraceStamps + (k)] = t_; } } while (0)
-#else
-#define RT_TT(k, extra) do { } while (0)
-#define RT_TG(k) do { } while (0)
-#endif
+// (profiles/r02_tail_phase_trace.txt).  128-thread CTAs, 3 per SM: 4 per SM spill more and were slower (DESIGN §5d).
+constexpr int kTailThreads = 128, kTailCtas = 3;
 template <bool kSmem, bool kBvh>
-__global__ void __launch_bounds__(kTailThreads, RT_TAIL_CTAS) k_bounce(const FastArgs a) {
+__global__ void __launch_bounds__(kTailThreads, kTailCtas) k_bounce(const FastArgs a) {
   extern __shared__ __align__(128) unsigned char smem[];
   // staged: [L light tables][general table], contiguous in global memory in that order
   const unsigned char *tabs = a.tabs + a.tstride;
@@ -1452,10 +1399,6 @@ __global__ void __launch_bounds__(kTailThreads, RT_TAIL_CTAS) k_bounce(const Fas
   // drain loops run for the slowest lane, and from kCoopMaxLive live rays down the tests turn lane-cooperative), 32 at most
   const unsigned nwarps = gridDim.x * (unsigned)(kTailThreads / 32);
   const unsigned per = min(32u, max(4u, (nq + nwarps - 1u) / nwarps));
-#ifdef RT_TAIL_TRACE
-  const unsigned tt_warp = blockIdx.x * (unsigned)(kTailThreads / 32) + (threadIdx.x >> 5);
-  bool tt_on = tt_warp < (unsigned)kTraceWarps;
-#endif
   for (;;) {
     const int chunk = warp_fetch(a.chunk_counter);
     if ((unsigned)chunk * per >= nq) break;
@@ -1477,10 +1420,8 @@ __global__ void __launch_bounds__(kTailThreads, RT_TAIL_CTAS) k_bounce(const Fas
       best_init(best[0]);
       // few live rays in this warp (the deep levels): the sphere tests run lane-cooperatively (coop_chunk_*)
       const bool coop = kSmem && !kBvh && __popc(__ballot_sync(kFull, live[0])) <= kCoopMaxLive;
-      RT_TT(0, __popc(__ballot_sync(kFull, live[0]))); RT_TG(6);
       if (kBvh) { if (live[0]) best[0] = bvh_closest_general(a, gen, ox[0], oy[0], oz[0], dx[0], dy[0], dz[0], src[0]); }
       else closest_general<1>(gen, a.npairs, a.N, ox, oy, oz, dx, dy, dz, live, a.d64, a.gS2, a.g_dtmax, a.r.sph64, src, best, coop);
-      RT_TT(1, 0);
       bool hit = false, final_ = false, cont = false;
       int idx[1] = {-1};
       double t64 = 0;
@@ -1506,7 +1447,6 @@ __global__ void __launch_bounds__(kTailThreads, RT_TAIL_CTAS) k_bounce(const Fas
           final_ = true;
         }
       }
-      RT_TT(2, __popc(__ballot_sync(kFull, hit)));
       // ---- shading of the hit (include/scene.h:89-121 in FP32, shadow booleans exact)
       d3 p = rtx::mk(0, 0, 0);
       float nx = 0.f, ny = 0.f, nz = 0.f, vx = 0.f, vy = 0.f, vz = 0.f, sr = 0.f, sg = 0.f, sb = 0.f, backthr = 0.f;
@@ -1522,10 +1462,6 @@ __global__ void __launch_bounds__(kTailThreads, RT_TAIL_CTAS) k_bounce(const Fas
         sr = g_frame.ambient[0] * m.x; sg = g_frame.ambient[1] * m.y; sb = g_frame.ambient[2] * m.z;
         backthr = -fmaxf(4.0f * kEps * rsqrtf((float)a.r.sph64[idx[0]].w), 1e-4f);          // -4 EPS / r (self-shadow shortcut, see k_shadow)
       }
-      RT_TT(3, 0);
-#ifdef RT_TAIL_TRACE
-      unsigned long long tt_prof[4] = {0ull, 0ull, 0ull, 0ull};
-#endif
       // ---- the shadow queries of the warp's hits: occm = occlusion bits of this lane's hit (bit l = light l)
       unsigned long long occm = 0ull;
       const unsigned hm = __ballot_sync(kFull, hit);
@@ -1582,11 +1518,7 @@ __global__ void __launch_bounds__(kTailThreads, RT_TAIL_CTAS) k_bounce(const Fas
             so = l2 * inv - kEps;
             cosl = -(qnx * sdx + qny * sdy + qnz * sdz);                        // n . light_dir
           }
-#ifdef RT_TAIL_TRACE
-          const bool o = shadow_mixed(tabs, a, l, sdx, sdy, sdz, so, act, qself, cosl, &pq.x, n_fp64, total <= kCoopMaxLive, tt_prof);
-#else
           const bool o = shadow_mixed(tabs, a, l, sdx, sdy, sdz, so, act, qself, cosl, &pq.x, n_fp64, total <= kCoopMaxLive);
-#endif
           const unsigned wm = __ballot_sync(kFull, act && o);
           for (int k = 0; taken != 0ull; k++) {          // this lane's queries of the round: list positions excl, excl + 1, ...
             const int l2 = __ffsll((long long)taken) - 1;
@@ -1627,11 +1559,6 @@ __global__ void __launch_bounds__(kTailThreads, RT_TAIL_CTAS) k_bounce(const Fas
         for (int l = 0; l < L; l++)
           if (!((occm >> l) & 1ull)) phong_light(l, p.x, p.y, p.z, nx, ny, nz, vx, vy, vz, m, mx.x, sr, sg, sb);
       }
-      RT_TT(4, 0);
-#ifdef RT_TAIL_TRACE
-      if (tt_on && lane == 0 && level - a.level < kTraceLevels)
-        for (int k = 0; k < 4; k++) g_tail_trace[(tt_warp * kTraceLevels + (level - a.level)) * kTraceStamps + 8 + k] = tt_prof[k];
-#endif
       // continuation: src/main.cpp:43-55 unrolled front to back
       if (hit) {
         if (a.r.shadow_mask) a.r.shadow_mask[(size_t)pix * a.r.max_depth + level] = smask;
@@ -1660,13 +1587,9 @@ __global__ void __launch_bounds__(kTailThreads, RT_TAIL_CTAS) k_bounce(const Fas
         if (lane == 0 && c_walks) { atomicAdd(&a.r.counters[RT_CNT_CAND], (unsigned long long)c_cand); atomicAdd(&a.r.counters[RT_CNT_WALKS], (unsigned long long)c_walks); }
         c_cand = c_walks = 0;
       }
-      RT_TT(5, __popc(__ballot_sync(kFull, cont))); RT_TG(7);
       live[0] = cont;
       if (!__any_sync(kFull, cont)) break;
     }
-#ifdef RT_TAIL_TRACE
-    tt_on = false;                                   // (first chunk of the warp only)
-#endif
   }
 }
 

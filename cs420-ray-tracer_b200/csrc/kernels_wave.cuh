@@ -25,15 +25,6 @@
 
 #include "kernels_fast.cuh"
 
-#ifndef RT_SHADOW_CTAS
-#define RT_SHADOW_CTAS 2
-#endif
-#ifndef RT_CLOSEST_CTAS
-#define RT_CLOSEST_CTAS 2
-#endif
-#ifndef RT_CLOSEST0_CTAS
-#define RT_CLOSEST0_CTAS RT_CLOSEST_CTAS
-#endif
 namespace rtf {
 
 // A camera-ray hit (level 0) has no queue record, carries weight 1 and no colour yet: there the words of (vy, vz), (src, wt)
@@ -148,13 +139,12 @@ __device__ __noinline__ int finish_hit(const FastArgs &a, Best b, RaySrc src, un
 
 // ---------------------------------------------------------------------------------------------
 // Table modes of the two table-walking kernels of level 0:
-//   kTabGlobal  tables read through L1/L2 (no staging)
 //   kTabSmem    the kernel's tables staged once per CTA with one TMA bulk copy (they fit)
 //   kTabStream  tables larger than shared memory: every CTA streams the (sorted) table through a
 //               two-stage ring of 32 KB tiles -- cp.async.bulk into stage k+1 while the eight warps
 //               test their rays against stage k (full barriers = mbarriers with expect_tx, the
 //               "stage is free again" edge = the CTA barrier that also votes on early termination).
-enum { kTabGlobal = 0, kTabSmem = 1, kTabStream = 2, kTabBvh = 3 };   // kTabBvh: candidates from the LBVH, tables in global memory
+enum { kTabSmem = 1, kTabStream = 2, kTabBvh = 3 };   // kTabBvh: candidates from the LBVH, tables in global memory
 constexpr int kTilePairs = 1024;                                   // sphere pairs per streamed tile
 constexpr unsigned kTileBytes = kTilePairs * 32u;                  // 32 KB per stage
 
@@ -270,8 +260,6 @@ __device__ __forceinline__ void closest0_body(const WaveArgs &w, unsigned char *
     const RaySrc src[2] = {{a.r.su, a.r.sv, x, j[0], nullptr}, {a.r.su, a.r.sv, x, j[1], nullptr}};
     if (kMode == kTabSmem) {
       closest_shared_culled<2>(cam, a.npairs, wb, dx, dy, dz, live, a.d64, a.r.sph64, src, best, c_cand, c_walks);
-    } else if (kMode == kTabGlobal) {
-      closest_shared<2>(cam, a.npairs, dx, dy, dz, live, a.d64, a.r.sph64, src, best);
     } else if (kMode == kTabBvh) {
       const float3 o = recentred(a, g_frame.cam_pos);
       // the tile's rays descend the hierarchy as ONE bundle; a per-ray traversal only if the bundle is too wide
@@ -386,8 +374,11 @@ __device__ __forceinline__ void closest0_body(const WaveArgs &w, unsigned char *
   }
   if (a.r.counters) flush_counts(a.r.counters, 0, c_closest, c_hits, 0, 0, c_fp64, c_viol, (unsigned long long)a.N, c_cand, c_walks, c_fall);
 }
+// 2 CTAs/SM (128 registers) for the table kernels k_closest0 / k_closest1 / k_shadow: more CTAs at fewer registers spill
+// and were slower (DESIGN §5d)
+constexpr int kTableCtas = 2;
 template <int kMode>
-__global__ void __launch_bounds__(kThreads, RT_CLOSEST0_CTAS) k_closest0(const WaveArgs w) {
+__global__ void __launch_bounds__(kThreads, kTableCtas) k_closest0(const WaveArgs w) {
   extern __shared__ __align__(128) unsigned char smem[];
   const FastArgs &a = w.f;
   const unsigned char *tabs = a.tabs;
@@ -471,7 +462,7 @@ __device__ __forceinline__ void closest1_body(const WaveArgs &w, const float4 *g
   if (a.r.counters) flush_counts(a.r.counters, level, c_closest, c_hits, 0, 0, c_fp64, c_viol, (unsigned long long)a.N, c_cand, c_walks);
 }
 template <bool kSmem, bool kBvh>
-__global__ void __launch_bounds__(kThreads, RT_CLOSEST_CTAS) k_closest1(const WaveArgs w) {
+__global__ void __launch_bounds__(kThreads, kTableCtas) k_closest1(const WaveArgs w) {
   extern __shared__ __align__(128) unsigned char smem[];
   const FastArgs &a = w.f;
   // staged: the general table only (it follows the (1+L) shared-origin tables)
@@ -636,12 +627,10 @@ __device__ __forceinline__ void shadow_body(const WaveArgs &w, unsigned char *sm
             if (!done && q.open[r]) occ[r] = bvh_shadow(a, T, o, l, dx[r], dy[r], dz[r], so[r], self[r], cosl[r], ppc[r], n64);
           }
         }
-      } else if (kMode != kTabStream) {
+      } else if (kMode == kTabSmem) {
         occ[0] = occ[1] = false;
-        if (__any_sync(kFull, want[0] || want[1])) {
-          if (kMode == kTabSmem) shadow_light_culled<2>(T, a.npairs, wb, l, dx, dy, dz, so, want, self, cosl, ppc, a.d64, a.r.sph64, occ, n64, c_cand, c_walks);
-          else shadow_light<2>(T, a.npairs, l, dx, dy, dz, so, want, self, cosl, ppc, a.d64, a.r.sph64, occ, n64);
-        }
+        if (__any_sync(kFull, want[0] || want[1]))
+          shadow_light_culled<2>(T, a.npairs, wb, l, dx, dy, dz, so, want, self, cosl, ppc, a.d64, a.r.sph64, occ, n64, c_cand, c_walks);
       } else {
         // the eight warps of the CTA walk this light's sorted table together, tile by tile
         const Tab TG = tab_at(gtabs, a, l);
@@ -722,7 +711,7 @@ __device__ __noinline__ void tile_offsets(unsigned int *tile_ray, int n, unsigne
 }
 
 template <int kMode>
-__global__ void __launch_bounds__(kThreads, RT_SHADOW_CTAS) k_shadow(const WaveArgs w) {
+__global__ void __launch_bounds__(kThreads, kTableCtas) k_shadow(const WaveArgs w) {
   extern __shared__ __align__(128) unsigned char smem[];
   const FastArgs &a = w.f;
   // staged: the L light tables
@@ -740,10 +729,8 @@ __global__ void __launch_bounds__(kThreads, RT_SHADOW_CTAS) k_shadow(const WaveA
 // CLOSEST HIT through the LBVH with DYNAMIC RAY FETCH (large scenes, reflection levels >= 1; see k_shadow_dyn for the
 // scheme).  Only the traversal runs here: a lane's result is the candidate bracket (Best) of its ray, stored per queued
 // ray; k_closest1 then does the exact finish for 64 neighbouring rays at a time, as before.
-#ifndef RT_DYN_CTAS
-#define RT_DYN_CTAS 4     // the traversal kernels are memory-latency bound: 64 registers / 32 warps per SM beat 97 / 16 (measured)
-#endif
-__global__ void __launch_bounds__(kThreads, RT_DYN_CTAS) k_closest1_dyn(const WaveArgs w) {
+constexpr int kDynCtas = 4;     // the traversal kernels are memory-latency bound: 64 registers / 32 warps per SM beat 97 / 16 (measured)
+__global__ void __launch_bounds__(kThreads, kDynCtas) k_closest1_dyn(const WaveArgs w) {
   const FastArgs &a = w.f;
   RT_PDL_SYNC();
   const unsigned nq = *a.q_in_count;
@@ -804,7 +791,7 @@ __global__ void __launch_bounds__(kThreads, RT_DYN_CTAS) k_closest1_dyn(const Wa
 // at 5-6 active lanes of 32 from reflection level 1 on), so here a lane does not wait for its warp: whenever enough
 // lanes are idle they fetch the next items together (one atomic per refill) and everybody goes on traversing
 // (persistent threads, Aila & Laine 2009).  Same queries, same slow paths, same occlusion bytes as k_shadow.
-__global__ void __launch_bounds__(kThreads, RT_DYN_CTAS) k_shadow_dyn(const WaveArgs w) {
+__global__ void __launch_bounds__(kThreads, kDynCtas) k_shadow_dyn(const WaveArgs w) {
   const FastArgs &a = w.f;
   RT_PDL_SYNC();
   const unsigned nh = *w.hit_count;
@@ -883,13 +870,6 @@ __global__ void __launch_bounds__(kThreads, RT_DYN_CTAS) k_shadow_dyn(const Wave
 // ---------------------------------------------------------------------------------------------
 // SHADE: one hit per lane.  include/scene.h:89-121 in FP32 with the occlusion bytes of k_shadow, then
 // src/main.cpp:43-55: final pixel, or the reflected ray (exact FP64) appended to the RayRec queue.
-#ifndef RT_SHADE_CTAS
-#define RT_SHADE_CTAS 4
-#endif
-#ifndef RT_SHADE_UNROLL
-#define RT_SHADE_UNROLL 1
-#endif
-constexpr int kShadeUnroll = RT_SHADE_UNROLL;   // 2: both halves of a hit block in one basic block (more loads in flight, more registers)
 __device__ __forceinline__ void prefetch_l1(const void *p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
 // a reflected ray of level 0 at its place in the tile-ordered queue (tile offset + rank); the capacity guard of queue_push
 __device__ __forceinline__ void queue_put(const WaveArgs &w, unsigned pos, const RayRec &rec) {
@@ -948,7 +928,7 @@ __device__ __forceinline__ void shade_body(const WaveArgs &w) {
         }
       }
       __syncwarp();
-#pragma unroll kShadeUnroll
+#pragma unroll 1
       for (int half = 0; half < 2; half++) {
         const unsigned h = blk * 64u + (unsigned)half * 32u + lane;
         const bool live = (h & 63u) < nslots && w.hits[h].idx >= 0;
@@ -1016,7 +996,8 @@ __device__ __forceinline__ void shade_body(const WaveArgs &w) {
   }
   if (a.r.counters) flush_counts(a.r.counters, 99, 0, 0, c_shadow, c_occ, 0, 0, (unsigned long long)a.N);
 }
-__global__ void __launch_bounds__(kThreads, RT_SHADE_CTAS) k_shade(const WaveArgs w) {
+constexpr int kShadeCtas = 4;   // memory-latency bound: 64 registers / 32 warps per SM
+__global__ void __launch_bounds__(kThreads, kShadeCtas) k_shade(const WaveArgs w) {
   RT_PDL_SYNC();
   shade_body(w);
 }

@@ -484,7 +484,7 @@ int rtk_fast_build_scene(RtFastScene *fs, const double *sph, int N, const RtFram
       const double E = 2.01 * std::ldexp(1.0, -20) * oc2 * (1 + 1e-9) + delta64;
       put(pairs, slot, (float)x, (float)y, (float)z, float_up(E - (oc2 - s[3] * s[3])));
       perm[slot] = i;
-      // bundle culling (kernels_fast.cuh, cull_round): unit vector to the centre, cos / sin of the angular radius
+      // bundle culling (kernels_fast.cuh, margins: see Cone): unit vector to the centre, cos / sin of the angular radius
       if (!lookup_only) {
         const double n = std::sqrt(oc2), r = std::fabs(s[3]) * (1.0 + 1e-6) + 1e-12;
         if (n > r * (1.0 + 1e-6)) {
@@ -982,14 +982,3 @@ double rtk_measure_fp32_peak(int device, double *sm_clock_mhz) {
   if (cudaGetLastError() != cudaSuccess) return -3;
   return 2.0 * grid * block * (double)iters * 16 * 8 / (best * 1e-3);
 }
-
-#ifdef RT_TAIL_TRACE
-// diagnostics build only: copies the tail kernel's phase stamps out (scripts/probe_tail_trace.py)
-extern "C" int rt_debug_tail_trace(unsigned long long *out, int n) {
-  const size_t total = sizeof(rtf::g_tail_trace);
-  const size_t want = (size_t)n * sizeof(unsigned long long);
-  if (cudaDeviceSynchronize() != cudaSuccess) return -1;
-  if (cudaMemcpyFromSymbol(out, rtf::g_tail_trace, want < total ? want : total) != cudaSuccess) return -1;
-  return (int)((want < total ? want : total) / sizeof(unsigned long long));
-}
-#endif

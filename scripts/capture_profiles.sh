@@ -30,10 +30,6 @@ if [ -n "$RT_CAPTURE_CSV" ]; then
 python scripts/benchmark_csv.py --iterations 2 --threads 1,4,16 --out $O/benchmark_results > $O/benchmark_csv.log 2>&1
 rm -f $O/benchmark_results/*.ppm
 fi
-# phase stamps of the tail kernel (diagnostics build of the same sources, scripts/build_variant.sh trace -DRT_TAIL_TRACE)
-if [ -f cs420-ray-tracer_b200/build/trace/librt_b200.so ]; then
-RTB200_LIB=cs420-ray-tracer_b200/build/trace/librt_b200.so timeout 120 python scripts/probe_tail_trace.py 1 8 > $O/tail_phase_trace.txt 2>&1
-fi
 timeout 200 python scripts/probe_depth2.py > $O/depth_increments.txt 2>&1
 python scripts/probe_e2e.py > $O/e2e_breakdown.log 2>&1
 ls -la $O

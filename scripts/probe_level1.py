@@ -3,9 +3,11 @@ and ms per frame of two builds of the library, alternated in one run.  Needs a B
 
   python scripts/probe_level1.py [--old LIB] [--new LIB] [--runs 3] [--out FILE]
 
-Each build is measured in its own process (RTB200_LIB); a build is made with scripts/build_variant.sh.  Per-kernel times
-come from torch.profiler with CUDA activities (a separate render loop of the same process; also for simple.txt at 1280x720
-d10, the workload whose tail consumes the level-0 queue directly); ms per frame from bench.py (profiler off).
+Each build is measured in its own process (RTB200_LIB).  A build outside the tree is made with
+  make -C cs420-ray-tracer_b200 BUILD=DIR LIB=DIR/librt_b200.so EXTRA_NVFLAGS=... DIR/librt_b200.so
+Per-kernel times come from torch.profiler with CUDA activities (a separate render loop of the same process; also for
+simple.txt at 1280x720 d10, the workload whose tail consumes the level-0 queue directly); ms per frame from bench.py
+(profiler off).
 
 Level-1 counters = those of a depth-2 render minus a depth-1 render, wave_levels 2, one context, three renders each.
 k_closest1 and k_shadow add into the same bundle_* counters; they are told apart with the same scene WITHOUT lights,
