@@ -36,17 +36,6 @@ namespace {
 constexpr size_t kMaxSmemTables = 90 * 1024;    // stage a kernel's tables in shared memory up to this size (2 CTAs/SM stay resident)
 constexpr int kCtlWords = rtf::CTL_WORDS;        // device control words per frame, layout: enum CTL_* (kernels_wave.cuh)
 
-inline float float_up(double x) {               // smallest float >= x
-  float f = (float)x;
-  if ((double)f < x) f = std::nextafterf(f, INFINITY);
-  return f;
-}
-inline float float_down(double x) {             // largest float <= x
-  float f = (float)x;
-  if ((double)f > x) f = std::nextafterf(f, -INFINITY);
-  return f;
-}
-
 #define RTK_TRY(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return -(int)e_; } while (0)
 
 }  // namespace
@@ -65,22 +54,13 @@ int rtk_fast_init(int) {
   return 0;
 }
 
-// Builds the FP32 filter tables on the host in double and rounds them conservatively
-// (DESIGN.md "filter margins"; error model in filter_math.cuh).
-//   shared-origin table for origin O (camera, each light), spheres SORTED by key = |oc| - r:
-//       oc = c_i - O (double -> nearest float), ncc = round_up(E_i - (|oc|^2 - r_i^2)),
-//       E_i = 2.01 * 2^-20 * |oc|^2 + delta64;  gmin[g] = round_down(key of the group's first sphere)
-//       perm[slot] = original sphere index (-1 = padding)
-//   general table (index order): c' = c_i - C0 (nearest float),
-//       rho' = round_up(r^2 (1+40u) + 12u S r + 64u^2 S^2 + delta64)
-// Sphere PAIRS are interleaved for the packed FP32x2 test: (x0,x1,y0,y1) (z0,z1,w0,w1).
 constexpr int RT_MAX_LEVELS_INTERNAL = 32;
 constexpr int kBvhAutoSpheres = 1024;   // automatic mode: scenes from this size on are traversed through the LBVH
 
 // Device build of the LBVH (bvh.cuh) over cen[i] = (c_i - C0, r_i) in FP32; eps inflates every box.
-// Inputs of the device LBVH build, written ON THE DEVICE from the raw sphere rows (large scenes: no host loop, no
-// host -> device copy of a second sphere array): cen[k] = (c - C0 in FP32, radius rounded up), orig[k] = sphere index, for
-// the spheres that are not in `big` (at most 8, ascending k keeps index order).
+// Inputs of the device LBVH build, written ON THE DEVICE from the raw sphere rows (no host loop, no host -> device copy
+// of a second sphere array): cen[k] = (c - C0 in FP32, radius rounded up), orig[k] = sphere index, for the spheres that
+// are not in `big` (at most 8, ascending k keeps index order).
 struct BuildBig { int n; int idx[8]; };
 __global__ void k_bvh_inputs(const double *__restrict__ raw, int N, double c0x, double c0y, double c0z, BuildBig big,
                              float4 *__restrict__ cen, int *__restrict__ orig) {
@@ -93,9 +73,9 @@ __global__ void k_bvh_inputs(const double *__restrict__ raw, int N, double c0x, 
   orig[i - before] = i;
 }
 
-// `cen` / `orig` host arrays, or nullptr + raw_dev: the inputs are produced on the device by k_bvh_inputs from the raw rows
-static int bvh_build(RtFastScene *fs, int n, const float4 *h_cen, const int *h_orig, const double *raw_dev, int N_all, const double *c0,
-                     const BuildBig &big, float eps, cudaStream_t stream) {
+// the inputs are produced on the device by k_bvh_inputs from the raw rows (raw_dev)
+static int bvh_build(RtFastScene *fs, int n, const double *raw_dev, int N_all, const double *c0, const BuildBig &big, float eps,
+                     cudaStream_t stream) {
   const int nleaf = (n + rtb::kLeafSize - 1) / rtb::kLeafSize, nint = nleaf > 1 ? nleaf - 1 : 1;
   // one scratch arena and the node array, both kept (grow-only) across uploads: cudaMalloc / cudaFree cost milliseconds
   // each once gigabytes of frame buffers are allocated, and a build needs seventeen arrays
@@ -128,12 +108,7 @@ static int bvh_build(RtFastScene *fs, int n, const float4 *h_cen, const int *h_o
       *flags = (int *)(sc + o_flags);
   fs->bvh_nodes = fs->bvh_nodes_buf;
   BV(cudaEventCreate(&e0)); BV(cudaEventCreate(&e1));
-  if (h_cen) {
-    BV(cudaMemcpyAsync(d_cen, h_cen, (size_t)n * 16, cudaMemcpyHostToDevice, stream));
-    BV(cudaMemcpyAsync(d_orig, h_orig, (size_t)n * 4, cudaMemcpyHostToDevice, stream));
-  } else {
-    k_bvh_inputs<<<(N_all + 255) / 256, 256, 0, stream>>>(raw_dev, N_all, c0[0], c0[1], c0[2], big, d_cen, d_orig);
-  }
+  k_bvh_inputs<<<(N_all + 255) / 256, 256, 0, stream>>>(raw_dev, N_all, c0[0], c0[1], c0[2], big, d_cen, d_orig);
   {
     const int init[6] = {0x7f7fffff, 0x7f7fffff, 0x7f7fffff, (int)0x80800000, (int)0x80800000, (int)0x80800000};   // ord(+max) / ord(-max)
     BV(cudaMemcpyAsync(bounds, init, sizeof(init), cudaMemcpyHostToDevice, stream));
@@ -146,8 +121,7 @@ static int bvh_build(RtFastScene *fs, int n, const float4 *h_cen, const int *h_o
     const int tb = 256, gb = (n + tb - 1) / tb, gl = (nleaf + tb - 1) / tb;
     rtb::k_bvh_bounds<<<gb < 592 ? gb : 592, tb, 0, stream>>>(d_cen, n, bounds);
     rtb::k_bvh_morton<<<gb, tb, 0, stream>>>(d_cen, n, bounds, keys[0], vals[0]);
-    const size_t sort_smem = (16 * rtb::kSortThreads + 32) * sizeof(unsigned);
-    BV(cudaFuncSetAttribute(rtb::k_bvh_sort, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sort_smem));
+    const size_t sort_smem = (16 * rtb::kSortThreads + 32) * sizeof(unsigned);   // (attribute set by rtk_fast_init)
     rtb::k_bvh_sort<<<1, rtb::kSortThreads, sort_smem, stream>>>(keys[0], vals[0], keys[1], vals[1], n, 8);   // 8 x 4 bits, result in [0]
     rtb::k_bvh_leaves<<<gl, tb, 0, stream>>>(d_cen, keys[0], vals[0], n, nleaf, eps, leaf_lo, leaf_hi, leaf_key);
     if (nleaf > 1) {
@@ -169,83 +143,171 @@ done:
   return rc;
 }
 
-// LOOKUP-ONLY tables (LBVH scenes) built on the device: one thread per (table, slot).  Slot order = sphere index, no
-// sort, no cull data (see lookup_only below); the same formulas and roundings as the host loop of build_table.
-struct BuildArgs {
-  const double *raw;          // N x 10 sphere rows (file column order), device
-  unsigned char *arena;       // tables | general table | ... (layout of RtFastScene)
-  double origin[RT_MAX_LIGHTS + 1][3];
-  int N, L, npairs, ngroups;
-  unsigned tstride, gmin_off, perm_off, inv_off;
-  size_t o_s64, o_mat, o_matx;
-  double delta64, c0[3], S, u;
-};
-__device__ __forceinline__ float dev_float_up(double x) { return __double2float_ru(x); }
-__device__ __forceinline__ void dev_put(float4 *pairs, int slot, float x, float y, float z, float w) {
-  float *A = reinterpret_cast<float *>(pairs + (size_t)(slot >> 1) * 2) + (slot & 1);
-  A[0] = x; A[2] = y; A[4] = z; A[6] = w;
+// ---------------------------------------------------------------------------------------------
+// The bytes of a table slot, defined once for the host build (sorted tables, at upload), k_cam_fill (the sorted camera
+// table, rt_set_camera) and k_build_lookup (lookup tables, at upload and rt_set_camera).  The FP32 filter tables are
+// computed in double and rounded conservatively (DESIGN.md "filter margins"; error model in filter_math.cuh):
+//   shared-origin table for origin O (camera, each light), spheres SORTED by key = |oc| - r (lookup layouts: index order):
+//       oc = c_i - O (double -> nearest float), w = round_up(E_i - (|oc|^2 - r_i^2)),
+//       E_i = 2.01 * 2^-20 * |oc|^2 + delta64;  gmin[g] = round_down(key of the group's first sphere)
+//       perm[slot] = original sphere index (-1 = padding)
+//   general table (index order): c' = c_i - C0 (nearest float),
+//       rho' = round_up(r^2 (1+40u) + 12u S r + 64u^2 S^2 + delta64)
+// Every double operation is one correctly rounded IEEE operation, in the same order on both sides, so host and device
+// write the same bytes.  On the device each is an explicit _rn intrinsic, which nvcc never contracts into an FMA; on the
+// host it is the plain operator, which stays one rounding only because NVFLAGS (Makefile) compile the host side with
+// -ffp-contract=off.  The conversions to float round to nearest, up or down, correctly on both sides.
+#ifdef __CUDA_ARCH__
+#define RT_RN(device, host) (device)
+#else
+#define RT_RN(device, host) (host)
+#endif
+namespace rn {
+inline float host_up(double x) {                // smallest float >= x
+  float f = (float)x;
+  if ((double)f < x) f = std::nextafterf(f, INFINITY);
+  return f;
 }
-__global__ void k_build_lookup(const BuildArgs b) {
-  const int slot = blockIdx.x * blockDim.x + threadIdx.x, t = blockIdx.y, nslots = 2 * b.npairs;
-  if (slot >= nslots) return;
-  if (t <= b.L) {                                      // shared-origin table t (camera, lights)
-    unsigned char *base = b.arena + (size_t)t * b.tstride;
-    float4 *pairs = reinterpret_cast<float4 *>(base);
-    int *perm = reinterpret_cast<int *>(base + b.perm_off), *inv = reinterpret_cast<int *>(base + b.inv_off);
-    float *gmin = reinterpret_cast<float *>(base + b.gmin_off);
-    if ((slot & 7) == 0) gmin[slot >> 3] = slot < b.N ? -3.0e38f : 3.0e38f;
-    if (slot >= b.N) { dev_put(pairs, slot, 0.f, 0.f, 0.f, -1.0f); perm[slot] = -1; return; }
-    const double *s = b.raw + (size_t)slot * 10;
-    const double x = __dsub_rn(s[0], b.origin[t][0]), y = __dsub_rn(s[1], b.origin[t][1]), z = __dsub_rn(s[2], b.origin[t][2]);
-    const double oc2 = __dadd_rn(__dadd_rn(__dmul_rn(x, x), __dmul_rn(y, y)), __dmul_rn(z, z)), r2 = __dmul_rn(s[3], s[3]);
-    const double E = 2.01 * 9.5367431640625e-07 * oc2 * (1 + 1e-9) + b.delta64;
-    dev_put(pairs, slot, (float)x, (float)y, (float)z, dev_float_up(E - (oc2 - r2)));
-    perm[slot] = slot;
-    inv[slot] = slot | ((oc2 - r2 > 1e-6 * (oc2 + r2) + 4.0 * b.delta64) ? 0x40000000 : 0);
-  } else {                                             // general table + exact geometry + materials
-    float4 *pairs = reinterpret_cast<float4 *>(b.arena + (size_t)(b.L + 1) * b.tstride);
-    if (slot >= b.N) { dev_put(pairs, slot, 0.f, 0.f, 0.f, -1.0e30f); return; }
-    const double *s = b.raw + (size_t)slot * 10;
-    const double r = fabs(s[3]);
-    const double rho = r * r * (1 + 40 * b.u) + 12 * b.u * b.S * r + 64 * b.u * b.u * b.S * b.S + b.delta64;
-    dev_put(pairs, slot, (float)(s[0] - b.c0[0]), (float)(s[1] - b.c0[1]), (float)(s[2] - b.c0[2]), dev_float_up(rho));
-    reinterpret_cast<double4 *>(b.arena + b.o_s64)[slot] = make_double4(s[0], s[1], s[2], __dmul_rn(s[3], s[3]));
-    reinterpret_cast<float4 *>(b.arena + b.o_mat)[slot] = make_float4((float)s[4], (float)s[5], (float)s[6], (float)s[7]);
-    reinterpret_cast<float2 *>(b.arena + b.o_matx)[slot] = make_float2((float)s[9], s[7] > 0 ? 1.0f : 0.0f);
+inline float host_down(double x) {              // largest float <= x
+  float f = (float)x;
+  if ((double)f > x) f = std::nextafterf(f, -INFINITY);
+  return f;
+}
+__host__ __device__ __forceinline__ double mul(double a, double b) { return RT_RN(__dmul_rn(a, b), a * b); }
+__host__ __device__ __forceinline__ double add(double a, double b) { return RT_RN(__dadd_rn(a, b), a + b); }
+__host__ __device__ __forceinline__ double sub(double a, double b) { return RT_RN(__dsub_rn(a, b), a - b); }
+__host__ __device__ __forceinline__ double div(double a, double b) { return RT_RN(__ddiv_rn(a, b), a / b); }
+__host__ __device__ __forceinline__ double sqrt(double a) { return RT_RN(__dsqrt_rn(a), std::sqrt(a)); }
+__host__ __device__ __forceinline__ float to_float(double a) { return RT_RN(__double2float_rn(a), (float)a); }
+__host__ __device__ __forceinline__ float up(double a) { return RT_RN(__double2float_ru(a), host_up(a)); }
+__host__ __device__ __forceinline__ float down(double a) { return RT_RN(__double2float_rd(a), host_down(a)); }
+}  // namespace rn
+#undef RT_RN
+
+// Sphere PAIRS are interleaved for the packed FP32x2 test: (x0,x1,y0,y1) (z0,z1,w0,w1).
+__host__ __device__ __forceinline__ void put_pair(float4 *pairs, int slot, float x, float y, float z, float w) {
+  float4 *A = pairs + (size_t)(slot >> 1) * 2, *B = A + 1;
+  if (slot & 1) { A->y = x; A->w = y; B->y = z; B->w = w; } else { A->x = x; A->z = y; B->x = z; B->z = w; }
+}
+
+// oc = c - O of a row (cx, cy, cz, r, ...), |oc|^2, and the sort key |oc| - |r|
+struct Oc { double x, y, z, oc2; };
+__host__ __device__ __forceinline__ Oc offset(const double *row, const double O[3]) {
+  Oc v;
+  v.x = rn::sub(row[0], O[0]); v.y = rn::sub(row[1], O[1]); v.z = rn::sub(row[2], O[2]);
+  v.oc2 = rn::add(rn::add(rn::mul(v.x, v.x), rn::mul(v.y, v.y)), rn::mul(v.z, v.z));
+  return v;
+}
+__host__ __device__ __forceinline__ double sort_key(const Oc &v, const double *row) { return rn::sub(rn::sqrt(v.oc2), fabs(row[3])); }
+
+// Byte layout of a shared-origin table (RtFastScene)
+struct TabLayout { unsigned tstride, gmin_off, perm_off, inv_off, cullA_off, cullB_off; };
+
+// Slot `slot` of the shared-origin table at `base` seen from O: sphere i with row[0..3] = (cx, cy, cz, r), or padding
+// when i < 0.  The slot heading a group also writes the group's gmin.  kSorted: a table sorted by key, with cull data
+// (table scenes); else a lookup table of an LBVH scene in index order without cull data (nothing walks it in order,
+// the hierarchy names the candidates).
+template <bool kSorted>
+__host__ __device__ __forceinline__ void shared_origin_slot(unsigned char *base, const TabLayout &t, int slot, int i, const double *row,
+                                                            const double O[3], double delta64) {
+  float4 *pairs = reinterpret_cast<float4 *>(base);
+  float *gmin = reinterpret_cast<float *>(base + t.gmin_off);
+  int *perm = reinterpret_cast<int *>(base + t.perm_off), *inv = reinterpret_cast<int *>(base + t.inv_off);
+  float4 *cullA = reinterpret_cast<float4 *>(base + t.cullA_off);
+  float *cullB = reinterpret_cast<float *>(base + t.cullB_off);
+  constexpr int kGroupSlots = 2 * rtf::kGroupPairs;
+  if (i < 0) {                                         // padding: never a candidate, always culled
+    put_pair(pairs, slot, 0.f, 0.f, 0.f, -1.0f); perm[slot] = -1;
+    if (kSorted) { cullA[slot] = make_float4(0.f, 0.f, 0.f, 4.0f); cullB[slot] = 0.f; }
+    if (slot % kGroupSlots == 0) gmin[slot / kGroupSlots] = 3.0e38f;
+    return;
+  }
+  const Oc v = offset(row, O);
+  const double r2 = rn::mul(row[3], row[3]);
+  const double E = rn::add(rn::mul(rn::mul(2.01 * 9.5367431640625e-07, v.oc2), 1 + 1e-9), delta64);
+  put_pair(pairs, slot, rn::to_float(v.x), rn::to_float(v.y), rn::to_float(v.z), rn::up(rn::sub(E, rn::sub(v.oc2, r2))));
+  perm[slot] = i;
+  // bit 30: the table origin (camera / light) is strictly outside sphere i, with a generous margin
+  inv[i] = slot | (rn::sub(v.oc2, r2) > rn::add(rn::mul(1e-6, rn::add(v.oc2, r2)), rn::mul(4.0, delta64)) ? 0x40000000 : 0);
+  if (kSorted) {
+    // bundle culling (kernels_fast.cuh, margins: see Cone): unit vector to the centre, cos / sin of the angular radius
+    const double n = rn::sqrt(v.oc2), r = rn::add(rn::mul(fabs(row[3]), 1.0 + 1e-6), 1e-12);
+    if (n > rn::mul(r, 1.0 + 1e-6)) {
+      const double sa = rn::div(r, n), ca = rn::sqrt(rn::mul(rn::sub(1.0, sa), rn::add(1.0, sa)));
+      cullA[slot] = make_float4(rn::to_float(rn::div(v.x, n)), rn::to_float(rn::div(v.y, n)), rn::to_float(rn::div(v.z, n)), rn::down(ca));
+      cullB[slot] = rn::up(sa);
+    } else {                                           // the origin is inside (or on) the sphere: never culled
+      cullA[slot] = make_float4(0.f, 0.f, 0.f, -4.0f); cullB[slot] = 0.f;
+    }
+  }
+  if (slot % kGroupSlots == 0) {                       // (index order: never a reason to stop)
+    const double k = sort_key(v, row);
+    gmin[slot / kGroupSlots] = kSorted ? rn::down(rn::sub(rn::sub(rn::sub(k, rn::mul(fabs(k), 1e-6)), 1e-6), delta64)) : -3.0e38f;
   }
 }
 
+// Slot i of the general table (index order, recentred by c0) and the exact geometry / material rows of sphere i, from
+// its row of 10 columns in file order; row == nullptr: a padding slot.
+__host__ __device__ __forceinline__ void general_slot(float4 *pairs, double4 *s64, float4 *mat, float2 *matx, int i, const double *row,
+                                                      const double c0[3], double S, double delta64) {
+  if (!row) { put_pair(pairs, i, 0.f, 0.f, 0.f, -1.0e30f); return; }
+  constexpr double u = 0x1p-24;
+  const double r = fabs(row[3]);
+  const double rho = rn::add(rn::add(rn::add(rn::mul(rn::mul(r, r), 1 + 40 * u), rn::mul(rn::mul(12 * u, S), r)),
+                                     rn::mul(rn::mul(rn::mul(64 * u, u), S), S)), delta64);
+  put_pair(pairs, i, rn::to_float(rn::sub(row[0], c0[0])), rn::to_float(rn::sub(row[1], c0[1])), rn::to_float(rn::sub(row[2], c0[2])),
+           rn::up(rho));
+  s64[i] = make_double4(row[0], row[1], row[2], rn::mul(row[3], row[3]));
+  mat[i] = make_float4(rn::to_float(row[4]), rn::to_float(row[5]), rn::to_float(row[6]), rn::to_float(row[7]));
+  matx[i] = make_float2(rn::to_float(row[9]), row[7] > 0 ? 1.0f : 0.0f);   // recurse flag decided in double
+}
+
+// The tables of LBVH scenes, written on the device from the raw rows: one thread per (table, slot).  blockIdx.y <= L:
+// the lookup table of origin y (camera, lights); L + 1: the general table, exact geometry and materials.
+struct BuildArgs {
+  const double *raw;          // N x 10 sphere rows (file column order), device
+  unsigned char *arena;       // tables | general table | ... (layout of RtFastScene)
+  double4 *s64;
+  float4 *mat;
+  float2 *matx;
+  TabLayout tab;
+  double origin[RT_MAX_LIGHTS + 1][3];
+  int N, L, nslots;
+  double delta64, c0[3], S;
+};
+__global__ void k_build_lookup(const BuildArgs b) {
+  const int slot = blockIdx.x * blockDim.x + threadIdx.x, t = blockIdx.y;
+  if (slot >= b.nslots) return;
+  const double *row = slot < b.N ? b.raw + (size_t)slot * 10 : nullptr;
+  if (t <= b.L)
+    shared_origin_slot<false>(b.arena + (size_t)t * b.tab.tstride, b.tab, slot, row ? slot : -1, row, b.origin[t], b.delta64);
+  else
+    general_slot(reinterpret_cast<float4 *>(b.arena + (size_t)(b.L + 1) * b.tab.tstride), b.s64, b.mat, b.matx, slot, row, b.c0, b.S,
+                 b.delta64);
+}
+
 // ---------------------------------------------------------------------------------------------
-// Camera table (table 0) rebuilt on the device for a new camera position (rt_set_camera), byte-identical to the host loop
-// of build_table(0, ...).  Every double operation is an explicit round-to-nearest intrinsic in the host's order of
-// evaluation (the host side is compiled with -ffp-contract=off; nvcc would otherwise contract a*b + c into an FMA), and
-// the host's (float) / float_up / float_down are __double2float_rn / _ru / _rd.  Input: geo[i] = (cx, cy, cz, r) as in
-// the file (r signed).
+// Sorted camera table (table 0) rebuilt on the device for a new camera position (rt_set_camera), byte-identical to the
+// host build.  Input: geo[i] = (cx, cy, cz, r) as in the file (r signed).
 //   k_cam_keys    key_i = sqrt(|c_i - O|^2) - |r_i| as an order-preserving 64-bit integer, split in two 32-bit words
 //   k_bvh_sort    (bvh.cuh) stable LSD radix sort on the low words, then on the high words gathered through the first
 //                 permutation (k_cam_gather): together the order of std::stable_sort on the doubles, ties by index
-//   k_cam_fill    pairs, perm, inv (bit 30), cullA / cullB and gmin from the sorted order; order == nullptr: index order
-//                 without cull data (the lookup-only tables of LBVH scenes)
+//   k_cam_fill    shared_origin_slot of every slot in the sorted order
 struct CamFillArgs {
   const double4 *geo;
   const int *order;
   unsigned char *base;        // table 0 = the start of the arena
-  int N, nslots, lookup_only;
-  unsigned gmin_off, perm_off, inv_off, cullA_off, cullB_off;
+  TabLayout tab;
+  int N, nslots;
   double O[3], delta64;
 };
-__device__ __forceinline__ double cam_key(const double4 g, double ox, double oy, double oz, double &x, double &y, double &z,
-                                          double &oc2) {
-  x = __dsub_rn(g.x, ox); y = __dsub_rn(g.y, oy); z = __dsub_rn(g.z, oz);
-  oc2 = __dadd_rn(__dadd_rn(__dmul_rn(x, x), __dmul_rn(y, y)), __dmul_rn(z, z));
-  return __dsub_rn(__dsqrt_rn(oc2), fabs(g.w));
-}
 __global__ void k_cam_keys(const double4 *__restrict__ geo, int N, double ox, double oy, double oz, unsigned *__restrict__ klo,
                            unsigned *__restrict__ khi, int *__restrict__ vals) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= N) return;
-  double x, y, z, oc2;
-  const double key = __dadd_rn(cam_key(geo[i], ox, oy, oz, x, y, z, oc2), 0.0);   // (-0 -> +0: the two compare equal)
+  const double4 g = geo[i];
+  const double row[4] = {g.x, g.y, g.z, g.w}, O[3] = {ox, oy, oz};
+  const double key = __dadd_rn(sort_key(offset(row, O), row), 0.0);   // (-0 -> +0: the two compare equal)
   unsigned long long u = (unsigned long long)__double_as_longlong(key);
   u = (u >> 63) ? ~u : (u | 0x8000000000000000ull);
   klo[i] = (unsigned)u; khi[i] = (unsigned)(u >> 32); vals[i] = i;
@@ -257,41 +319,11 @@ __global__ void k_cam_gather(const unsigned *__restrict__ src, const int *__rest
 __global__ void k_cam_fill(const CamFillArgs b) {
   const int slot = blockIdx.x * blockDim.x + threadIdx.x;
   if (slot >= b.nslots) return;
-  float4 *pairs = reinterpret_cast<float4 *>(b.base);
-  float *gmin = reinterpret_cast<float *>(b.base + b.gmin_off);
-  int *perm = reinterpret_cast<int *>(b.base + b.perm_off), *inv = reinterpret_cast<int *>(b.base + b.inv_off);
-  float4 *cullA = reinterpret_cast<float4 *>(b.base + b.cullA_off);
-  float *cullB = reinterpret_cast<float *>(b.base + b.cullB_off);
-  constexpr int kGroupSlots = 2 * rtf::kGroupPairs;
-  if (slot >= b.N) {                                   // padding: never a candidate, always culled
-    if (slot % kGroupSlots == 0) gmin[slot / kGroupSlots] = 3.0e38f;
-    dev_put(pairs, slot, 0.f, 0.f, 0.f, -1.0f); perm[slot] = -1;
-    if (!b.lookup_only) { cullA[slot] = make_float4(0.f, 0.f, 0.f, 4.0f); cullB[slot] = 0.f; }
-    return;
-  }
-  const int i = b.order ? b.order[slot] : slot;
+  if (slot >= b.N) { shared_origin_slot<true>(b.base, b.tab, slot, -1, nullptr, b.O, b.delta64); return; }
+  const int i = b.order[slot];
   const double4 g = b.geo[i];
-  double x, y, z, oc2;
-  const double key = cam_key(g, b.O[0], b.O[1], b.O[2], x, y, z, oc2);
-  const double r2 = __dmul_rn(g.w, g.w);
-  const double E = __dadd_rn(__dmul_rn(__dmul_rn(2.01 * 9.5367431640625e-07, oc2), 1 + 1e-9), b.delta64);
-  dev_put(pairs, slot, __double2float_rn(x), __double2float_rn(y), __double2float_rn(z), __double2float_ru(__dsub_rn(E, __dsub_rn(oc2, r2))));
-  perm[slot] = i;
-  if (!b.lookup_only) {
-    const double n = __dsqrt_rn(oc2), r = __dadd_rn(__dmul_rn(fabs(g.w), 1.0 + 1e-6), 1e-12);
-    if (n > __dmul_rn(r, 1.0 + 1e-6)) {
-      const double sa = __ddiv_rn(r, n), ca = __dsqrt_rn(__dmul_rn(__dsub_rn(1.0, sa), __dadd_rn(1.0, sa)));
-      cullA[slot] = make_float4(__double2float_rn(__ddiv_rn(x, n)), __double2float_rn(__ddiv_rn(y, n)), __double2float_rn(__ddiv_rn(z, n)),
-                                __double2float_rd(ca));
-      cullB[slot] = __double2float_ru(sa);
-    } else {                                           // the origin is inside (or on) the sphere: never culled
-      cullA[slot] = make_float4(0.f, 0.f, 0.f, -4.0f); cullB[slot] = 0.f;
-    }
-  }
-  inv[i] = slot | ((__dsub_rn(oc2, r2) > __dadd_rn(__dmul_rn(1e-6, __dadd_rn(oc2, r2)), __dmul_rn(4.0, b.delta64))) ? 0x40000000 : 0);
-  if (slot % kGroupSlots == 0)
-    gmin[slot / kGroupSlots] = b.lookup_only ? -3.0e38f
-                                             : __double2float_rd(__dsub_rn(__dsub_rn(__dsub_rn(key, __dmul_rn(fabs(key), 1e-6)), 1e-6), b.delta64));
+  const double row[4] = {g.x, g.y, g.z, g.w};
+  shared_origin_slot<true>(b.base, b.tab, slot, i, row, b.O, b.delta64);
 }
 
 // Per-column / per-row camera-plane coordinates (include/camera.h:18-22, src/main.cpp:151-152) in the operation order of
@@ -313,6 +345,26 @@ int rtk_camera_plane(double *su, int nu, double *sv, int nv, int m, int W, int H
   k_cam_plane<<<(n + 255) / 256, 256, 0, stream>>>(su, nu, sv, nv, m, W, H, scale);
   const cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? 0 : -(int)e;
+}
+
+static TabLayout tab_layout(const RtFastScene *fs) {
+  return {fs->tstride, fs->gmin_off, fs->perm_off, fs->inv_off, fs->cullA_off, fs->cullB_off};
+}
+
+// k_build_lookup's arguments for the lookup tables of fs: table 0 seen from cam_pos, tables 1..L from light_pos, the
+// general table recentred with the extent bound S.  rt_set_camera rebuilds table 0 only and passes no lights and no S.
+static BuildArgs lookup_args(const RtFastScene *fs, const double cam_pos[3], const double (*light_pos)[3], double S) {
+  BuildArgs b;
+  memset(&b, 0, sizeof(b));
+  b.raw = (const double *)fs->raw_dev; b.arena = (unsigned char *)fs->tabs;
+  b.s64 = (double4 *)fs->sph64; b.mat = (float4 *)fs->mat; b.matx = (float2 *)fs->matx;
+  b.tab = tab_layout(fs);
+  for (int k = 0; k < 3; k++) { b.origin[0][k] = cam_pos[k]; b.c0[k] = fs->c0[k]; }
+  if (light_pos)
+    for (int l = 0; l < fs->L; l++) for (int k = 0; k < 3; k++) b.origin[l + 1][k] = light_pos[l][k];
+  b.N = fs->N; b.L = fs->L; b.nslots = 2 * fs->npairs;
+  b.delta64 = fs->delta64; b.S = S;
+  return b;
 }
 
 int rtk_fast_build_scene(RtFastScene *fs, const double *sph, int N, const RtFrameConst *f, int accel, cudaStream_t stream) {
@@ -351,7 +403,7 @@ int rtk_fast_build_scene(RtFastScene *fs, const double *sph, int N, const RtFram
   fs->sabs_scene = sabs;
   const double delta64 = rtk_delta64(sabs, f->cam_pos);
   fs->delta64 = delta64;
-  fs->d64 = float_up(delta64);
+  fs->d64 = rn::up(delta64);
   for (int k = 0; k < 3; k++) fs->c0[k] = N > 0 ? 0.5 * (lo[k] + hi[k]) : 0.0;
   double S = 0;
   for (int i = 0; i < N; i++) {
@@ -360,17 +412,15 @@ int rtk_fast_build_scene(RtFastScene *fs, const double *sph, int N, const RtFram
     S = std::fmax(S, std::sqrt(x * x + y * y + z * z) + std::fabs(s[3]));
   }
   S += 0.01;
-  fs->gS2 = float_up(S * S * 1.0001);
-  fs->g_dtmax = float_up(80.0 * u * S);
+  fs->gS2 = rn::up(S * S * 1.0001);
+  fs->g_dtmax = rn::up(80.0 * u * S);
 
   // LBVH scenes: the candidates of every query come from the hierarchy, the tables are only LOOKED UP by sphere (inv ->
   // slot -> pair); nothing walks them in order, prunes by gmin or culls by cone.  So they keep index order -- no sort
-  // (five stable sorts of 100 k keys were most of a config-5 upload) -- and carry no cull data; from kDeviceBuildSpheres
-  // spheres on they are written by a kernel from the raw rows (k_build_lookup) instead of staged on the host.
+  // (five stable sorts of 100 k keys were most of a config-5 upload) -- and carry no cull data, and a kernel writes them
+  // from the raw rows (k_build_lookup) instead of staging them on the host.
   const bool lookup_only = N > 0 && (accel == 2 || (accel == 0 && N >= kBvhAutoSpheres));
-  constexpr int kDeviceBuildSpheres = 2048;
-  const bool device_build = lookup_only && N >= kDeviceBuildSpheres;
-  fs->lookup_only = lookup_only; fs->device_build = device_build;
+  fs->lookup_only = lookup_only;
   // byte layout of one shared-origin table
   const unsigned pairs_bytes = (unsigned)npairs * 32u;
   const unsigned gmin_bytes = ((unsigned)ngroups * 4u + 15u) & ~15u;
@@ -383,32 +433,22 @@ int rtk_fast_build_scene(RtFastScene *fs, const double *sph, int N, const RtFram
   // stride = 32 (mod 128) bytes: when the lanes of a warp walk DIFFERENT lights' tables in step (shadow_mixed), the same
   // pair of four consecutive tables lies in four different bank groups of shared memory
   fs->tstride += (32u + 128u - fs->tstride % 128u) % 128u;
-  fs->bytes_primary = (size_t)(L + 1) * fs->tstride;
   fs->bytes_bounce = (size_t)L * fs->tstride + pairs_bytes;
   const size_t total = (size_t)(L + 1) * fs->tstride + pairs_bytes;
-  // arena = tables | sph64 | mat | matx | geo, staged in one pinned buffer (grow-only).  geo = (cx, cy, cz, r) per sphere:
-  // the input of the device rebuild of the camera table (rtk_fast_camera_table); device-built scenes read raw_dev instead
+  // arena = tables | sph64 | mat | matx | geo in one device allocation (grow-only).  geo = (cx, cy, cz, r) per sphere, sorted
+  // layouts only: the input of the device rebuild of the camera table (rtk_fast_camera_table); lookup layouts read raw_dev
   const size_t n1 = (size_t)(N > 0 ? N : 1);
   const size_t o_s64 = (total + 255) & ~(size_t)255, o_mat = o_s64 + n1 * sizeof(double4), o_matx = o_mat + n1 * sizeof(float4);
   const size_t o_geo = ((o_matx + n1 * sizeof(float2)) + 255) & ~(size_t)255;
-  const size_t arena = ((o_geo + n1 * sizeof(double4)) + 255) & ~(size_t)255;
+  const size_t arena = lookup_only ? o_geo : ((o_geo + n1 * sizeof(double4)) + 255) & ~(size_t)255;
   if (fs->tabs_cap < arena) {
     cudaFree(fs->tabs); fs->tabs = nullptr; fs->tabs_cap = 0;
     RTK_TRY(cudaMalloc(&fs->tabs, arena));
     fs->tabs_cap = arena;
   }
   fs->sph64 = (unsigned char *)fs->tabs + o_s64; fs->mat = (unsigned char *)fs->tabs + o_mat; fs->matx = (unsigned char *)fs->tabs + o_matx;
-  fs->geo = device_build ? nullptr : (unsigned char *)fs->tabs + o_geo;
-  // scratch of the camera-table sort (keys: 3 x N words, values: 2 x N), grow-only: rt_set_camera allocates nothing
-  if (!lookup_only) {
-    const size_t need = 5 * (((size_t)N * 4 + 255) & ~(size_t)255);
-    if (fs->cam_scratch_cap < need) {
-      cudaFree(fs->cam_scratch); fs->cam_scratch = nullptr; fs->cam_scratch_cap = 0;
-      RTK_TRY(cudaMalloc(&fs->cam_scratch, need));
-      fs->cam_scratch_cap = need;
-    }
-  }
-  if (device_build) {
+  fs->geo = lookup_only ? nullptr : (unsigned char *)fs->tabs + o_geo;
+  if (lookup_only) {
     const size_t raw_bytes = (size_t)N * 10 * sizeof(double);
     if (fs->raw_cap < raw_bytes) {
       cudaFree(fs->raw_dev); fs->raw_dev = nullptr; fs->raw_cap = 0;
@@ -416,120 +456,66 @@ int rtk_fast_build_scene(RtFastScene *fs, const double *sph, int N, const RtFram
       fs->raw_cap = raw_bytes;
     }
     RTK_TRY(cudaMemcpyAsync(fs->raw_dev, sph, raw_bytes, cudaMemcpyHostToDevice, stream));
-    BuildArgs b;
-    memset(&b, 0, sizeof(b));
-    b.raw = (const double *)fs->raw_dev; b.arena = (unsigned char *)fs->tabs;
-    for (int k = 0; k < 3; k++) { b.origin[0][k] = f->cam_pos[k]; b.c0[k] = fs->c0[k]; }
-    for (int l = 0; l < L; l++) for (int k = 0; k < 3; k++) b.origin[l + 1][k] = f->light_pos[l][k];
-    b.N = N; b.L = L; b.npairs = npairs; b.ngroups = ngroups;
-    b.tstride = fs->tstride; b.gmin_off = fs->gmin_off; b.perm_off = fs->perm_off; b.inv_off = fs->inv_off;
-    b.o_s64 = o_s64; b.o_mat = o_mat; b.o_matx = o_matx; b.delta64 = delta64; b.S = S; b.u = u;
+    RTK_TRY(cudaMemsetAsync(fs->tabs, 0, total, stream));   // the gaps of the layout, as the host build clears them
+    const BuildArgs b = lookup_args(fs, f->cam_pos, f->light_pos, S);
     k_build_lookup<<<dim3((unsigned)(nslots + 255) / 256, (unsigned)(L + 2)), 256, 0, stream>>>(b);
     RTK_TRY(cudaGetLastError());
   } else {
-  if (fs->h_stage_cap < arena) {
-    if (fs->h_stage) cudaFreeHost(fs->h_stage);
-    fs->h_stage = nullptr; fs->h_stage_cap = 0;
-    RTK_TRY(cudaHostAlloc(&fs->h_stage, arena, cudaHostAllocDefault));
-    fs->h_stage_cap = arena;
-  }
-  struct { unsigned char *p; unsigned char *data() const { return p; } } h = {(unsigned char *)fs->h_stage};
-  memset(h.p, 0, total);
-  {
-    double4 *s64 = reinterpret_cast<double4 *>(h.p + o_s64);
-    float4 *mat = reinterpret_cast<float4 *>(h.p + o_mat);
-    float2 *matx = reinterpret_cast<float2 *>(h.p + o_matx);
-    double4 *geo = reinterpret_cast<double4 *>(h.p + o_geo);
-    for (int i = 0; i < N; i++) {
-      const double *r = sph + (size_t)i * 10;
-      geo[i] = make_double4(r[0], r[1], r[2], r[3]);
-      s64[i] = make_double4(r[0], r[1], r[2], r[3] * r[3]);
-      mat[i] = make_float4((float)r[4], (float)r[5], (float)r[6], (float)r[7]);
-      matx[i] = make_float2((float)r[9], r[7] > 0 ? 1.0f : 0.0f);   // recurse flag decided in double
+    // scratch of the camera-table sort (keys: 3 x N words, values: 2 x N), grow-only: rt_set_camera allocates nothing
+    const size_t need = 5 * (((size_t)N * 4 + 255) & ~(size_t)255);
+    if (fs->cam_scratch_cap < need) {
+      cudaFree(fs->cam_scratch); fs->cam_scratch = nullptr; fs->cam_scratch_cap = 0;
+      RTK_TRY(cudaMalloc(&fs->cam_scratch, need));
+      fs->cam_scratch_cap = need;
+    }
+    if (fs->h_stage_cap < arena) {
+      if (fs->h_stage) cudaFreeHost(fs->h_stage);
+      fs->h_stage = nullptr; fs->h_stage_cap = 0;
+      RTK_TRY(cudaHostAlloc(&fs->h_stage, arena, cudaHostAllocDefault));
+      fs->h_stage_cap = arena;
+    }
+    unsigned char *h = (unsigned char *)fs->h_stage;
+    memset(h, 0, total);
+    const TabLayout tab = tab_layout(fs);
+    std::vector<int> order((size_t)(N > 0 ? N : 1));
+    std::vector<double> key((size_t)(N > 0 ? N : 1));
+    auto build_table = [&](int t, std::vector<int> &order, std::vector<double> &key) {
+      const double *O = t == 0 ? f->cam_pos : f->light_pos[t - 1];
+      for (int i = 0; i < N; i++) {
+        const double *s = sph + (size_t)i * 10;
+        key[i] = sort_key(offset(s, O), s);
+        order[i] = i;
+      }
+      std::stable_sort(order.begin(), order.begin() + N, [&](int p, int q) { return key[p] < key[q]; });
+      for (int slot = 0; slot < nslots; slot++) {
+        const int i = slot < N ? order[slot] : -1;
+        shared_origin_slot<true>(h + (size_t)t * fs->tstride, tab, slot, i, i < 0 ? nullptr : sph + (size_t)i * 10, O, delta64);
+      }
+    };
+    // the (1+L) tables are independent: large scenes build them on separate host threads
+    if (N >= 4096 && L >= 1) {
+      std::vector<std::thread> th;
+      for (int t = 0; t <= L; t++)
+        th.emplace_back([&, t]() { std::vector<int> o2((size_t)N); std::vector<double> k2((size_t)N); build_table(t, o2, k2); });
+      for (auto &x : th) x.join();
+    } else {
+      for (int t = 0; t <= L; t++) build_table(t, order, key);
+    }
+    float4 *gen = reinterpret_cast<float4 *>(h + (size_t)(L + 1) * fs->tstride);
+    double4 *s64 = reinterpret_cast<double4 *>(h + o_s64), *geo = reinterpret_cast<double4 *>(h + o_geo);
+    float4 *mat = reinterpret_cast<float4 *>(h + o_mat);
+    float2 *matx = reinterpret_cast<float2 *>(h + o_matx);
+    for (int i = 0; i < nslots; i++) {
+      const double *s = i < N ? sph + (size_t)i * 10 : nullptr;
+      general_slot(gen, s64, mat, matx, i, s, fs->c0, S, delta64);
+      if (s) geo[i] = make_double4(s[0], s[1], s[2], s[3]);
     }
     if (N == 0) { s64[0] = make_double4(0, 0, 0, 0); mat[0] = make_float4(0, 0, 0, 0); matx[0] = make_float2(0, 0); }
+    RTK_TRY(cudaMemcpyAsync(fs->tabs, h, arena, cudaMemcpyHostToDevice, stream));
   }
-  auto put = [&](float4 *pairs, int slot, float x, float y, float z, float w) {
-    float4 *A = pairs + (size_t)(slot >> 1) * 2, *B = A + 1;
-    if (slot & 1) { A->y = x; A->w = y; B->y = z; B->w = w; } else { A->x = x; A->z = y; B->x = z; B->z = w; }
-  };
-  std::vector<int> order((size_t)(N > 0 ? N : 1));
-  std::vector<double> key((size_t)(N > 0 ? N : 1));
-  auto build_table = [&](int t, std::vector<int> &order, std::vector<double> &key) {
-    unsigned char *base = h.data() + (size_t)t * fs->tstride;
-    float4 *pairs = reinterpret_cast<float4 *>(base);
-    float *gmin = reinterpret_cast<float *>(base + fs->gmin_off);
-    int *perm = reinterpret_cast<int *>(base + fs->perm_off);
-    int *inv = reinterpret_cast<int *>(base + fs->inv_off);
-    float4 *cullA = reinterpret_cast<float4 *>(base + fs->cullA_off);
-    float *cullB = reinterpret_cast<float *>(base + fs->cullB_off);
-    const double *O = t == 0 ? f->cam_pos : f->light_pos[t - 1];
-    for (int i = 0; i < N; i++) {
-      const double *s = sph + (size_t)i * 10;
-      const double x = s[0] - O[0], y = s[1] - O[1], z = s[2] - O[2];
-      key[i] = std::sqrt(x * x + y * y + z * z) - std::fabs(s[3]);
-      order[i] = i;
-    }
-    if (!lookup_only) std::stable_sort(order.begin(), order.begin() + N, [&](int p, int q) { return key[p] < key[q]; });
-    for (int slot = 0; slot < nslots; slot++) {
-      if (slot >= N) {                                 // padding: never a candidate, always culled
-        put(pairs, slot, 0.f, 0.f, 0.f, -1.0f); perm[slot] = -1;
-        cullA[slot] = make_float4(0.f, 0.f, 0.f, 4.0f); cullB[slot] = 0.f;
-        continue;
-      }
-      const int i = order[slot];
-      const double *s = sph + (size_t)i * 10;
-      const double x = s[0] - O[0], y = s[1] - O[1], z = s[2] - O[2];
-      const double oc2 = x * x + y * y + z * z;
-      const double E = 2.01 * std::ldexp(1.0, -20) * oc2 * (1 + 1e-9) + delta64;
-      put(pairs, slot, (float)x, (float)y, (float)z, float_up(E - (oc2 - s[3] * s[3])));
-      perm[slot] = i;
-      // bundle culling (kernels_fast.cuh, margins: see Cone): unit vector to the centre, cos / sin of the angular radius
-      if (!lookup_only) {
-        const double n = std::sqrt(oc2), r = std::fabs(s[3]) * (1.0 + 1e-6) + 1e-12;
-        if (n > r * (1.0 + 1e-6)) {
-          const double sa = r / n, ca = std::sqrt((1.0 - sa) * (1.0 + sa));
-          cullA[slot] = make_float4((float)(x / n), (float)(y / n), (float)(z / n), float_down(ca));
-          cullB[slot] = float_up(sa);
-        } else {                                       // the origin is inside (or on) the sphere: never culled
-          cullA[slot] = make_float4(0.f, 0.f, 0.f, -4.0f); cullB[slot] = 0.f;
-        }
-      }
-      // bit 30: the table origin (camera / light) is strictly outside sphere i, with a generous margin
-      inv[i] = slot | ((oc2 - s[3] * s[3] > 1e-6 * (oc2 + s[3] * s[3]) + 4.0 * delta64) ? 0x40000000 : 0);
-    }
-    for (int g = 0; g < ngroups; g++) {
-      const int slot = g * 2 * rtf::kGroupPairs;
-      if (slot >= N) { gmin[g] = 3.0e38f; continue; }
-      if (lookup_only) { gmin[g] = -3.0e38f; continue; }   // (unsorted: never a reason to stop)
-      const double k = key[order[slot]];
-      gmin[g] = float_down(k - std::fabs(k) * 1e-6 - 1e-6 - delta64);
-    }
-  };
-  // the (1+L) tables are independent: large scenes build them on separate host threads
-  if (N >= 4096 && L >= 1) {
-    std::vector<std::thread> th;
-    for (int t = 0; t <= L; t++)
-      th.emplace_back([&, t]() { std::vector<int> o2((size_t)N); std::vector<double> k2((size_t)N); build_table(t, o2, k2); });
-    for (auto &x : th) x.join();
-  } else {
-    for (int t = 0; t <= L; t++) build_table(t, order, key);
-  }
-  {
-    float4 *pairs = reinterpret_cast<float4 *>(h.data() + (size_t)(L + 1) * fs->tstride);
-    for (int i = 0; i < nslots; i++) {
-      if (i >= N) { put(pairs, i, 0.f, 0.f, 0.f, -1.0e30f); continue; }
-      const double *s = sph + (size_t)i * 10;
-      const double r = std::fabs(s[3]);
-      const double rho = r * r * (1 + 40 * u) + 12 * u * S * r + 64 * u * u * S * S + delta64;
-      put(pairs, i, (float)(s[0] - fs->c0[0]), (float)(s[1] - fs->c0[1]), (float)(s[2] - fs->c0[2]), float_up(rho));
-    }
-  }
-  RTK_TRY(cudaMemcpyAsync(fs->tabs, h.data(), arena, cudaMemcpyHostToDevice, stream));
-  }   // host build
   RTK_TRY(cudaStreamSynchronize(stream));   // the staging buffer / the caller's sphere rows may be reused from here on
-  fs->bvh_nodes = fs->bvh_leaves = nullptr; fs->bvh_nleaf = 0; fs->bvh_build_ms = 0; fs->nbig = 0;
-  if (N > 0 && (accel == 2 || (accel == 0 && N >= kBvhAutoSpheres))) {
+  fs->bvh_nodes = nullptr; fs->bvh_nleaf = 0; fs->bvh_build_ms = 0; fs->nbig = 0;
+  if (lookup_only) {
     // Spheres far larger than the typical one (a ground sphere ...) stay out of the hierarchy: their boxes would make
     // every ancestor cover the scene, so every ray would walk that whole root-to-leaf path.  They are tested per ray.
     std::vector<double> rad((size_t)N);
@@ -545,26 +531,12 @@ int rtk_fast_build_scene(RtFastScene *fs, const double *sph, int N, const RtFram
     for (int k = 0; k < fs->nbig; k++) fs->big[k] = bigs[k];
     // box inflation: FP32 rounding of recentred centres / ray origins (<= u S each) and the 12u direction error over
     // any distance <= 2S inside the scene ball, with a 2x reserve: 64u * 3S
-    const float eps = float_up(64.0 * u * 3.0 * S);
+    const float eps = rn::up(64.0 * u * 3.0 * S);
     BuildBig big;
     memset(&big, 0, sizeof(big));
     big.n = fs->nbig;
     for (int k = 0; k < fs->nbig; k++) big.idx[k] = fs->big[k];
-    int r;
-    if (device_build) {
-      r = bvh_build(fs, N - fs->nbig, nullptr, nullptr, (const double *)fs->raw_dev, N, fs->c0, big, eps, stream);
-    } else {
-      std::vector<float4> cen;
-      std::vector<int> orig;
-      cen.reserve((size_t)N); orig.reserve((size_t)N);
-      for (int i = 0; i < N; i++) {
-        if (std::find(bigs.begin(), bigs.end(), i) != bigs.end()) continue;
-        const double *s = sph + (size_t)i * 10;
-        cen.push_back(make_float4((float)(s[0] - fs->c0[0]), (float)(s[1] - fs->c0[1]), (float)(s[2] - fs->c0[2]), float_up(rad[i])));
-        orig.push_back(i);
-      }
-      r = bvh_build(fs, (int)cen.size(), cen.data(), orig.data(), nullptr, N, fs->c0, big, eps, stream);
-    }
+    const int r = bvh_build(fs, N - fs->nbig, (const double *)fs->raw_dev, N, fs->c0, big, eps, stream);
     if (r != 0) return r;
   }
   return 0;
@@ -578,38 +550,28 @@ double rtk_delta64(double sabs_scene, const double cam_pos[3]) {
 int rtk_fast_camera_table(RtFastScene *fs, const double cam_pos[3], cudaStream_t stream) {
   const int N = fs->N, nslots = 2 * fs->npairs, tb = 256;
   if (N == 0) return 0;                                // (padding only: nothing depends on the camera)
-  if (fs->device_build) {
-    // the table-0 half of the kernel that built it at upload: the same code, so the same bytes
-    BuildArgs b;
-    memset(&b, 0, sizeof(b));
-    b.raw = (const double *)fs->raw_dev; b.arena = (unsigned char *)fs->tabs;
-    for (int k = 0; k < 3; k++) { b.origin[0][k] = cam_pos[k]; b.c0[k] = fs->c0[k]; }
-    b.N = N; b.L = fs->L; b.npairs = fs->npairs; b.ngroups = fs->ngroups;
-    b.tstride = fs->tstride; b.gmin_off = fs->gmin_off; b.perm_off = fs->perm_off; b.inv_off = fs->inv_off;
-    b.delta64 = fs->delta64;
-    k_build_lookup<<<dim3((unsigned)(nslots + tb - 1) / tb, 1u), tb, 0, stream>>>(b);
+  if (fs->lookup_only) {
+    // table 0 of the kernel that built the tables at upload
+    k_build_lookup<<<dim3((unsigned)(nslots + tb - 1) / tb, 1u), tb, 0, stream>>>(lookup_args(fs, cam_pos, nullptr, 0.0));
     RTK_TRY(cudaGetLastError());
     return 0;
   }
   CamFillArgs a;
   memset(&a, 0, sizeof(a));
-  a.geo = (const double4 *)fs->geo; a.base = (unsigned char *)fs->tabs;
-  a.N = N; a.nslots = nslots; a.lookup_only = fs->lookup_only;
-  a.gmin_off = fs->gmin_off; a.perm_off = fs->perm_off; a.inv_off = fs->inv_off; a.cullA_off = fs->cullA_off; a.cullB_off = fs->cullB_off;
+  a.geo = (const double4 *)fs->geo; a.base = (unsigned char *)fs->tabs; a.tab = tab_layout(fs);
+  a.N = N; a.nslots = nslots;
   for (int k = 0; k < 3; k++) a.O[k] = cam_pos[k];
   a.delta64 = fs->delta64;
-  if (!fs->lookup_only) {
-    const size_t w = ((size_t)N * 4 + 255) & ~(size_t)255;
-    unsigned char *sc = (unsigned char *)fs->cam_scratch;
-    unsigned *k0 = (unsigned *)sc, *k1 = (unsigned *)(sc + w), *k2 = (unsigned *)(sc + 2 * w);
-    int *v0 = (int *)(sc + 3 * w), *v1 = (int *)(sc + 4 * w);
-    const size_t sort_smem = (16 * rtb::kSortThreads + 32) * sizeof(unsigned);
-    k_cam_keys<<<(N + tb - 1) / tb, tb, 0, stream>>>(a.geo, N, cam_pos[0], cam_pos[1], cam_pos[2], k0, k2, v0);
-    rtb::k_bvh_sort<<<1, rtb::kSortThreads, sort_smem, stream>>>(k0, v0, k1, v1, N, 8);   // low words; result in (k0, v0)
-    k_cam_gather<<<(N + tb - 1) / tb, tb, 0, stream>>>(k2, v0, k1, N);
-    rtb::k_bvh_sort<<<1, rtb::kSortThreads, sort_smem, stream>>>(k1, v0, k0, v1, N, 8);   // high words; order in v0
-    a.order = v0;
-  }
+  const size_t w = ((size_t)N * 4 + 255) & ~(size_t)255;
+  unsigned char *sc = (unsigned char *)fs->cam_scratch;
+  unsigned *k0 = (unsigned *)sc, *k1 = (unsigned *)(sc + w), *k2 = (unsigned *)(sc + 2 * w);
+  int *v0 = (int *)(sc + 3 * w), *v1 = (int *)(sc + 4 * w);
+  const size_t sort_smem = (16 * rtb::kSortThreads + 32) * sizeof(unsigned);
+  k_cam_keys<<<(N + tb - 1) / tb, tb, 0, stream>>>(a.geo, N, cam_pos[0], cam_pos[1], cam_pos[2], k0, k2, v0);
+  rtb::k_bvh_sort<<<1, rtb::kSortThreads, sort_smem, stream>>>(k0, v0, k1, v1, N, 8);   // low words; result in (k0, v0)
+  k_cam_gather<<<(N + tb - 1) / tb, tb, 0, stream>>>(k2, v0, k1, N);
+  rtb::k_bvh_sort<<<1, rtb::kSortThreads, sort_smem, stream>>>(k1, v0, k0, v1, N, 8);   // high words; order in v0
+  a.order = v0;
   k_cam_fill<<<(nslots + tb - 1) / tb, tb, 0, stream>>>(a);
   RTK_TRY(cudaGetLastError());
   return 0;
@@ -626,7 +588,7 @@ void rtk_fast_free_scene(RtFastScene *fs, int release_tables) {
     fs->bvh_nodes_buf = fs->bvh_scratch = nullptr; fs->bvh_nodes_cap = fs->bvh_scratch_cap = 0;
     fs->raw_dev = nullptr; fs->raw_cap = 0;
   }
-  fs->bvh_nodes = fs->bvh_leaves = nullptr; fs->bvh_nleaf = 0;
+  fs->bvh_nodes = nullptr; fs->bvh_nleaf = 0;
 }
 
 // The error word of the last frame launched (call after the stream has been synchronised): bounds guards of the hit /

@@ -15,16 +15,15 @@ int rtk_launch_exact(const RtRenderArgs &args, cudaStream_t stream);
 // mode 0: FP32-filter fast path (kernels_fast.cuh).
 struct RtFastScene {
   int N, L, npairs, ngroups;
-  void *tabs;             // device: (1+L) shared-origin tables (pairs | gmin | perm), then the general table
+  void *tabs;             // device: (1+L) shared-origin tables (pairs | gmin | perm | inv [| cullA | cullB]), then the general table
   size_t tabs_cap;        // bytes allocated behind tabs (reused by the next upload when large enough)
   // the exact geometry / materials live in the same device arena, behind the tables: ONE pinned staging buffer and ONE
   // host->device copy per upload
   void *sph64, *mat, *matx;   // device: N x double4, N x float4, N x float2
-  void *h_stage; size_t h_stage_cap;   // pinned host staging of the whole arena
-  void *raw_dev; size_t raw_cap;       // large LBVH scenes: the raw sphere rows on the device (tables are built there)
+  void *h_stage; size_t h_stage_cap;   // pinned host staging of the whole arena (sorted layouts)
+  void *raw_dev; size_t raw_cap;       // LBVH scenes: the raw sphere rows on the device (tables and LBVH are built there)
   unsigned tstride;       // bytes per shared-origin table
   unsigned gmin_off, perm_off, inv_off, cullA_off, cullB_off;
-  size_t bytes_primary;   // staged by k_primary: (1+L) * tstride
   size_t bytes_bounce;    // staged by k_bounce : L * tstride + npairs * 32
   float d64;              // absolute FP64/geometry slack (delta64)
   float gS2;              // squared radius bound of the recentred scene
@@ -32,7 +31,7 @@ struct RtFastScene {
   unsigned long long generation;   // bumped by every rtk_fast_build_scene
   double c0[3];           // recentring offset of the general table
   // device-built LBVH over the recentred spheres (bvh.cuh); built when the scene has >= bvh_min spheres
-  void *bvh_nodes, *bvh_leaves;   // bvh_nodes = bvh_nodes_buf when the current scene has a hierarchy, else NULL
+  void *bvh_nodes;        // bvh_nodes_buf when the current scene has a hierarchy, else NULL
   void *bvh_nodes_buf, *bvh_scratch;   // grow-only allocations kept across uploads
   size_t bvh_nodes_cap, bvh_scratch_cap;
   int bvh_nleaf;
@@ -41,8 +40,8 @@ struct RtFastScene {
   // camera moves without a re-upload (rtk_fast_camera_table): what the upload decided and kept for it
   double sabs_scene;      // magnitude bound of the lights and spheres, without the camera
   double delta64;         // the slack the tables were built with (fs->d64 is its float rounding)
-  int lookup_only, device_build;   // table layout: index-order lookup tables (LBVH scenes); written by k_build_lookup
-  void *geo;              // device, inside the arena: N x double4 (cx, cy, cz, r); NULL when device_build (raw_dev)
+  int lookup_only;        // table layout: index-order lookup tables without cull data (LBVH scenes), written by k_build_lookup
+  void *geo;              // device, inside the arena: N x double4 (cx, cy, cz, r) of sorted layouts; NULL for lookup layouts (raw_dev)
   void *cam_scratch; size_t cam_scratch_cap;   // sort scratch of the camera table (sorted layouts), grow-only
 };
 struct RtFastWork {

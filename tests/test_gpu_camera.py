@@ -96,7 +96,7 @@ def test_orbit_sorted_tables_of_synthetic_scenes(rt, n):
 
 
 @gpu
-@pytest.mark.parametrize("n", [1500, 2100])       # LBVH scenes: lookup tables built on the host / on the device (>= 2048)
+@pytest.mark.parametrize("n", [1500, 2100])       # LBVH scenes, lookup tables (k_build_lookup): on both sides of 2048 spheres, where a host build used to end
 def test_orbit_lookup_tables_of_lbvh_scenes(rt, n):
     sc = synth(rt, n)
     follow(rt, sc, orbit(sc.camera, 8, turn=1.0))
