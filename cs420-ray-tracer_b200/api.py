@@ -23,7 +23,7 @@ ABI_SYMBOLS = [
     "rt_host_alloc", "rt_host_free", "rt_write_ppm", "rt_measure_fp32_peak",
     "rt_create_multi", "rt_multi_destroy", "rt_multi_ranks", "rt_multi_ctx", "rt_multi_set_option", "rt_multi_upload_scene",
     "rt_multi_render", "rt_render_bands_host", "rt_host_register", "rt_host_unregister",
-    "rt_set_camera", "rt_multi_set_camera",
+    "rt_set_camera", "rt_multi_set_camera", "rt_multi_render_path",
 ]
 
 
@@ -112,6 +112,7 @@ def load_library():
     lib.rt_multi_set_option.argtypes = [vp, C.c_char_p, C.c_longlong]
     lib.rt_multi_upload_scene.argtypes = [vp, vp, i, vp, i, vp, vp, vp, C.c_double]
     lib.rt_multi_render.argtypes = [vp, i, i, i, i, vp, C.POINTER(RtStats)]
+    lib.rt_multi_render_path.argtypes = [vp, vp, i, i, i, i, vp, vp]
     lib.rt_render_bands_host.argtypes = [vp, i, i, i, i, i, i, vp, C.POINTER(RtStats)]
     lib.rt_host_register.argtypes = [vp, C.c_size_t]
     lib.rt_host_unregister.argtypes = [vp]
@@ -199,6 +200,22 @@ def host_register(ptr, nbytes):
 
 def host_unregister(ptr):
     _check(load_library().rt_host_unregister(C.c_void_p(ptr)), "rt_host_unregister")
+
+
+def _path_args(cameras, W, H, device, out):
+    """(cameras as K x 7 float64, the uint8 [K, H, W, 3] output on cuda:device, torch's current stream there) of a
+    camera-path render."""
+    import torch
+    cams = np.ascontiguousarray(cameras, dtype=np.float64).reshape(-1, 7)
+    dev = torch.device("cuda", device)
+    K = cams.shape[0]
+    if out is None:
+        out = torch.empty((K, H, W, 3), dtype=torch.uint8, device=dev)
+    if tuple(out.shape) != (K, H, W, 3) or out.dtype != torch.uint8 or out.device != dev or not out.is_contiguous():
+        raise RtError("render_path: out must be a contiguous uint8 [%d, %d, %d, 3] tensor on %s" % (K, H, W, dev))
+    # (torch's legacy default stream is handle 0, which the library reads as "the ctx stream": pass cudaStreamLegacy)
+    stream = torch.cuda.current_stream(dev).cuda_stream or 1
+    return cams, out, stream
 
 
 def band_rows(H, band_h, rank, nranks):
@@ -328,15 +345,9 @@ class Renderer:
         on this renderer's device, row 0 = bottom.  Every frame is rt_set_camera + rt_render_bands on torch's current
         stream, with no host synchronisation between frames; the camera of the last row stays set."""
         import torch
-        cams = np.ascontiguousarray(cameras, dtype=np.float64).reshape(-1, 7)
-        dev = torch.device("cuda", self.device)
+        cams, out, stream = _path_args(cameras, W, H, self.device, out)
+        dev = out.device
         K = cams.shape[0]
-        if out is None:
-            out = torch.empty((K, H, W, 3), dtype=torch.uint8, device=dev)
-        if tuple(out.shape) != (K, H, W, 3) or out.dtype != torch.uint8 or out.device != dev or not out.is_contiguous():
-            raise RtError("render_path: out must be a contiguous uint8 [%d, %d, %d, 3] tensor on %s" % (K, H, W, dev))
-        # (torch's legacy default stream is handle 0, which the library reads as "the ctx stream": pass cudaStreamLegacy)
-        stream = torch.cuda.current_stream(dev).cuda_stream or 1
         # the kernels store 16-byte row segments: a frame that does not start 16-byte aligned goes through a staging frame
         stage = None if (H * W * 3) % 16 == 0 else torch.empty((H, W, 3), dtype=torch.uint8, device=dev)
         with torch.cuda.device(dev):
@@ -400,7 +411,8 @@ class Renderer:
 
 class MultiRenderer:
     """rt_create_multi: one frame sharded by interleaved row bands over `ngpus` ranks inside this process; every rank
-    copies its bands to the host frame over its own link."""
+    copies its bands to the host frame over its own link.  render_path instead gives whole frames of a camera path to
+    the ranks."""
 
     def __init__(self, ngpus, mode="fast", accel=None):
         self._lib = load_library()
@@ -436,6 +448,15 @@ class MultiRenderer:
         _check(self._lib.rt_multi_render(self._h, W, H, depth, band_h, out.ctypes.data, C.byref(st) if want_stats else None),
                "rt_multi_render")
         return out, st
+
+    def render_path(self, cameras, W, H, depth, out=None):
+        """rt_multi_render_path: one frame per camera row (px py pz lx ly lz fov), rank k % n renders frame k, as a torch
+        uint8 [K, H, W, 3] tensor on rank 0's device (cuda:0), row 0 = bottom, ordered on torch's current stream there
+        (no host synchronisation).  The frames equal Renderer.render_path's; every rank keeps the last camera set."""
+        cams, out, stream = _path_args(cameras, W, H, 0, out)
+        _check(self._lib.rt_multi_render_path(self._h, cams.ctypes.data, cams.shape[0], W, H, depth, C.c_void_p(out.data_ptr()),
+                                              C.c_void_p(stream)), "rt_multi_render_path")
+        return out
 
     def close(self):
         if getattr(self, "_h", None):

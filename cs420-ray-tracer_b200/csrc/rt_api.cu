@@ -688,6 +688,10 @@ struct rt_multi {
   int n = 0;
   std::vector<rt_ctx *> ctx;
   void *registered = nullptr; size_t registered_bytes = 0;   // host frame pinned by us (cudaHostRegister) for async copies
+  // rt_multi_render_path: ev_in on rank 0's device (the caller's stream at the call), ev_done[r] on rank r's device (its
+  // last frame copy)
+  cudaEvent_t ev_in = nullptr;
+  std::vector<cudaEvent_t> ev_done;
 };
 
 extern "C" void rt_multi_destroy(rt_multi *m) {
@@ -696,6 +700,8 @@ extern "C" void rt_multi_destroy(rt_multi *m) {
     if (!m->ctx[r]) continue;
     cudaSetDevice(m->ctx[r]->device);
     cudaStreamSynchronize(m->ctx[r]->stream);
+    if (r < (int)m->ev_done.size() && m->ev_done[r]) cudaEventDestroy(m->ev_done[r]);
+    if (r == 0 && m->ev_in) cudaEventDestroy(m->ev_in);
     rt_destroy(m->ctx[r]);
   }
   if (m->registered) cudaHostUnregister(m->registered);
@@ -711,11 +717,19 @@ extern "C" int rt_create_multi(int ngpus, rt_multi **out) {
   if (!m) return rt_fail(RT_ERR_NOMEM, "rt_create_multi: out of memory");
   m->n = ngpus;
   m->ctx.assign((size_t)ngpus, nullptr);
+  m->ev_done.assign((size_t)ngpus, nullptr);
   for (int r = 0; r < ngpus; r++) {
     // more ranks than devices: ranks share devices round robin (same frame, no speed-up) -- lets a 1-GPU box run the
     // N-rank code path
     const int rc = rt_create(r % ndev, &m->ctx[r]);
     if (rc != RT_OK) { const std::string msg = g_last_error; rt_multi_destroy(m); return rt_fail(rc, msg); }
+    // (rt_create left the rank's device current)
+    cudaError_t e = cudaEventCreateWithFlags(&m->ev_done[r], cudaEventDisableTiming);
+    if (e == cudaSuccess && r == 0) e = cudaEventCreateWithFlags(&m->ev_in, cudaEventDisableTiming);
+    if (e != cudaSuccess) {
+      rt_multi_destroy(m);
+      return rt_fail(RT_ERR_CUDA, std::string("rt_create_multi: ") + cudaGetErrorString(e));
+    }
   }
   *out = m;
   return RT_OK;
@@ -798,5 +812,99 @@ extern "C" int rt_multi_render(rt_multi *m, int W, int H, int depth, int band_h,
     *stats = acc;
     stats->ms_host = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   }
+  return RT_OK;
+}
+
+// ---- a camera path frame-parallel over the ranks ---------------------------------------------------------------------
+// One frame of rt_multi_render_path on rank c: rt_set_camera + a full-frame render into the ctx's own frame buffer (the
+// kernels store 16-byte row segments, so they never write the caller's frames directly), then one copy to `dst` on
+// rank 0's device (peer memory unless c lives there).  wait_first: the first frame of the rank waits for the caller's
+// stream before its copy, so the rendering itself overlaps the caller's earlier work.
+static int path_frame(rt_ctx *c, const double *cam, int W, int H, int depth, uint8_t *dst, cudaEvent_t wait_first) {
+  int rc = rt_set_camera(c, cam, cam + 3, cam[6], nullptr);
+  if (rc) return rc;
+  const size_t bytes = (size_t)W * H * 3;
+  RT_CUDA(cudaSetDevice(c->device));
+  if ((rc = ensure_cap(c->d_rgb, c->rgb_cap, bytes + 16))) return rc;
+  if ((rc = render_common(c, W, H, depth, H, 0, 1, c->d_rgb, nullptr, nullptr, c->stream, nullptr))) return rc;
+  if (wait_first) RT_CUDA(cudaStreamWaitEvent(c->stream, wait_first, 0));
+  RT_CUDA(cudaMemcpyAsync(dst, c->d_rgb, bytes, cudaMemcpyDeviceToDevice, c->stream));
+  return RT_OK;
+}
+
+extern "C" int rt_multi_render_path(rt_multi *m, const double *cameras, int K, int W, int H, int depth, void *dev_frames,
+                                    void *stream) {
+  if (!m || !cameras || !dev_frames) return rt_fail(RT_ERR_ARG, "rt_multi_render_path: NULL argument");
+  if (K < 1 || W < 1 || H < 1 || depth < 0) return rt_fail(RT_ERR_ARG, "rt_multi_render_path: bad frame count, image size or depth");
+  const int n = m->n, dev0 = m->ctx[0]->device;
+  for (int r = 0; r < n; r++)
+    if (!m->ctx[r]->have_scene) return rt_fail(RT_ERR_STATE, "rt_multi_render_path: no scene uploaded (call rt_multi_upload_scene first)");
+  cudaPointerAttributes pa;
+  RT_CUDA(cudaPointerGetAttributes(&pa, dev_frames));
+  if (pa.type != cudaMemoryTypeDevice || pa.device != dev0)
+    return rt_fail(RT_ERR_ARG, "rt_multi_render_path: dev_frames must be device memory of rank 0's device " + std::to_string(dev0));
+  // the devices in rank order; ranks that share a device are enqueued by one thread, because the device's __constant__
+  // bank changes hands between its contexts in the order their renders are enqueued (render_common), which needs one order
+  std::vector<int> devs;
+  for (int r = 0; r < n; r++) {
+    const int d = m->ctx[r]->device;
+    bool seen = false;
+    for (int x : devs) seen |= x == d;
+    if (seen) continue;
+    devs.push_back(d);
+    if (d == dev0) continue;
+    // the ranks copy their frames into rank 0's memory: peer access, enabled on demand; no staging through the host
+    int can = 0;
+    RT_CUDA(cudaDeviceCanAccessPeer(&can, d, dev0));
+    if (!can)
+      return rt_fail(RT_ERR_UNSUPPORTED, "rt_multi_render_path: device " + std::to_string(d) + " has no peer access to device " +
+                                             std::to_string(dev0));
+    RT_CUDA(cudaSetDevice(d));
+    const cudaError_t e = cudaDeviceEnablePeerAccess(dev0, 0);
+    if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+    else if (e != cudaSuccess) return rt_fail(RT_ERR_CUDA, std::string("rt_multi_render_path: cudaDeviceEnablePeerAccess: ") + cudaGetErrorString(e));
+  }
+  const cudaStream_t s0 = stream ? (cudaStream_t)stream : m->ctx[0]->stream;
+  RT_CUDA(cudaSetDevice(dev0));
+  RT_CUDA(cudaEventRecord(m->ev_in, s0));
+
+  const size_t bytes = (size_t)W * H * 3;
+  const double *last = cameras + (size_t)(K - 1) * 7;
+  std::vector<int> rc((size_t)n, RT_OK);
+  std::vector<std::string> msg((size_t)n);
+  std::vector<char> wrote((size_t)n, 0);              // the rank's stream waited for ev_in: `stream` must wait for it
+  auto one_device = [&](int dev) {
+    int bad = -1, e = RT_OK;
+    for (int k = 0; k < K && e == RT_OK; k++) {       // rank k % n renders frame k
+      const int r = k % n;
+      if (m->ctx[r]->device != dev) continue;
+      const bool first = !wrote[r];
+      wrote[r] = 1;
+      e = path_frame(m->ctx[r], cameras + (size_t)k * 7, W, H, depth, (uint8_t *)dev_frames + (size_t)k * bytes,
+                     first ? m->ev_in : nullptr);
+      if (e != RT_OK) bad = r;
+    }
+    for (int r = 0; r < n; r++) {
+      if (m->ctx[r]->device != dev) continue;
+      if (wrote[r]) {                                 // (also after a failure: `stream` waits for whatever was enqueued)
+        const cudaError_t ce = cudaEventRecord(m->ev_done[r], m->ctx[r]->stream);
+        if (ce != cudaSuccess && e == RT_OK) { e = rt_fail(RT_ERR_CUDA, std::string("rt_multi_render_path: cudaEventRecord: ") + cudaGetErrorString(ce)); bad = r; }
+      }
+      // every rank ends on the last camera, as Renderer.render_path does
+      if (e == RT_OK && r != (K - 1) % n && (e = rt_set_camera(m->ctx[r], last, last + 3, last[6], nullptr)) != RT_OK) bad = r;
+    }
+    if (bad >= 0) { rc[bad] = e; msg[bad] = g_last_error; }   // (thread local: copy it out of the worker thread)
+  };
+  if (devs.size() == 1) one_device(devs[0]);
+  else {
+    std::vector<std::thread> th;
+    for (int d : devs) th.emplace_back(one_device, d);
+    for (auto &t : th) t.join();
+  }
+  // `stream` waits on the device for every frame copy; also after a failure, so that no copy outlives the caller's buffer
+  RT_CUDA(cudaSetDevice(dev0));
+  for (int r = 0; r < n; r++)
+    if (wrote[r]) RT_CUDA(cudaStreamWaitEvent(s0, m->ev_done[r], 0));
+  for (int r = 0; r < n; r++) if (rc[r] != RT_OK) return rt_fail(rc[r], msg[r]);
   return RT_OK;
 }

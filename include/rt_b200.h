@@ -226,6 +226,26 @@ int rt_multi_upload_scene(rt_multi *m, const double *spheres, int nspheres, cons
 int rt_multi_set_camera(rt_multi *m, const double cam_pos[3], const double cam_look[3], double fov_deg);
 int rt_multi_render(rt_multi *m, int width, int height, int max_depth, int band_h, uint8_t *host_rgb,
                     rt_stats *stats);
+/* A camera path frame-parallel over the ranks: whole frames go to different GPUs instead of every frame being split into
+ * bands, so each GPU renders full frames at its single-GPU efficiency.  cameras: K rows of 7 host doubles, px py pz lx ly
+ * lz fov (the scene file's order).  dev_frames: K*H*W*3 bytes of device memory on RANK 0's device; frame k starts at
+ * k*H*W*3 (any alignment), row 0 = bottom.  Rank k % ngpus renders frame k exactly as rt_set_camera with cameras[k]
+ * followed by a full-frame render on that rank would, so every frame is byte-identical to the same path rendered on one
+ * context with the same options (mode, accel, antialias, wave_levels).  A rank renders into a frame buffer on its own
+ * device and copies it into place (a peer copy from another device; peer access is enabled on demand, and a device pair
+ * without it is RT_ERR_UNSUPPORTED -- nothing is staged through host memory).
+ * Asynchronous: every rank works on its ctx stream, in that ctx's render order, and the host enqueues the ranks' frames
+ * on parallel threads (one per device; ranks that share a device share one), joined before the call returns.  No
+ * frame is written before the work already on `stream` at the call has finished, and `stream` waits, on the device, for
+ * every frame: the caller consumes them on `stream` without a host synchronisation.  `stream` is a cudaStream_t of rank
+ * 0's device passed as void* (NULL = rank 0's ctx stream).  The one host synchronisation is rt_set_camera's: a camera
+ * that leaves the extent of the lights and spheres (or comes back inside it) makes that rank rebuild its scene and wait.
+ * Afterwards every rank's camera is cameras[K-1].  There is no rt_stats argument: per-frame counters would need a host
+ * synchronisation per frame.  RT_ERR_ARG for a NULL pointer, K < 1, a size below 1, max_depth < 0 or dev_frames not on
+ * rank 0's device; RT_ERR_STATE before rt_multi_upload_scene; when ranks fail, the error of the lowest failing rank,
+ * after every thread has joined.  With more ranks than devices the frames are the same, without a speed-up.        */
+int rt_multi_render_path(rt_multi *m, const double *cameras, int K, int width, int height, int max_depth,
+                         void *dev_frames, void *stream);
 
 /* One process per GPU (torchrun): as rt_multi_render's per-rank half.  Every rank calls it with the SAME host frame
  * (shared memory, W*H*3 bytes, row 0 = bottom) and its own (rank, nranks); the rank's bands are rendered and copied to
